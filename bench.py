@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — DDIM-50 makeup images/s at 256^2 (BASELINE.json metric), per the driver contract.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" = one pass of the hot path over one batch: 50-step DDIM sampling (eta 0, no CFG) of a batch of
@@ -36,6 +36,24 @@ sys.path.insert(0, ROOT)
 # algorithmic FLOPs (SURVEY.md §8(d)): per sample per step excluding step-invariant work, and once per sample
 F_STEP = {256: 234.788e9, 512: 1067.53e9}
 F_ONCE = {256: 8.052e9, 512: 19.26e9}
+DUMP_BYTES = 63 * 10**6  # --dump-outputs: data of all arrays together, so that the files with their headers stay under 64 MB
+
+
+def dump_outputs(out_dir, arrays, budget=DUMP_BYTES):
+    """Writes every tensor of `arrays` as out_dir/<name>.npy in float32.  When together they hold more than `budget`
+    bytes, each keeps the same share of its flattened elements: a sample drawn with a fixed seed and kept in index
+    order, so that runs with the same arguments write the same elements and two builds compare element for element."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    total = 4 * sum(a.numel() for a in arrays.values())
+    for name, a in arrays.items():
+        a = a.detach().float().cpu()
+        if total > budget:
+            pick = torch.randperm(a.numel(), generator=torch.Generator().manual_seed(0))[:a.numel() * budget // total]
+            a = a.flatten()[pick.sort().values]
+        np.save(os.path.join(out_dir, f"{name}.npy"), a.numpy())
+        print(f"bench: wrote {name}.npy {tuple(a.shape)} to {out_dir}" + (" (sample)" if total > budget else ""), file=sys.stderr)
 
 
 def peaks():
@@ -114,7 +132,7 @@ class OracleCPU:
     def run(self, n):
         with self.torch.no_grad():
             t0 = time.perf_counter()
-            self.s.reconstruct(self.x, self.cond, t_start=n, **self.guide)  # the first n steps of the schedule
+            self.out = self.s.reconstruct(self.x, self.cond, t_start=n, **self.guide)  # the first n steps of the schedule
             return time.perf_counter() - t0
 
 
@@ -156,6 +174,8 @@ def reference_arm(args, rank):
         o.run(1)
     full_s = o.run(S)
     times = [o.run(n) for _ in range(args.steps)]
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"latents": o.out})
     sec_per_model_step = statistics.mean(times) / n
     ips = 1.0 / (S * sec_per_model_step)
     cores = o.cores
@@ -212,7 +232,14 @@ def main():
                          "c_crossattn, DDIM, first-stage decode, uint8 image grid (mkd_image_grid_u8) -> host; implies --decode; "
                          "off by default (not BASELINE.json's metric) and named in config.workload when on")
     ap.add_argument("--profile-out", default=None, help="write the per-layer kernel timing table to this file")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one returned on rank 0 (the final latents, or the decoded "
+                         "images with --decode) as DIR/<name>.npy in float32, at most 64 MB in all (beyond that a fixed "
+                         "seeded sample of the elements); the inputs depend only on the arguments, so two builds compare "
+                         "output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank, world = int(os.environ.get("RANK", 0)), int(os.environ.get("WORLD_SIZE", 1))
     local = int(os.environ.get("LOCAL_RANK", 0))
     if args.impl == "reference":
@@ -359,27 +386,30 @@ def main():
         torch.cuda.synchronize()
 
     def timed(fn, k):
+        """k passes of fn between two events: (milliseconds, max over ranks; what the last pass returned)"""
         barrier()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for _ in range(k):
-            fn()
+            out = fn()
         e1.record()
         barrier()
         ms = torch.tensor([e0.elapsed_time(e1)], device=dev)
         if world > 1:
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
-        return float(ms)
+        return float(ms), out
 
     for _ in range(args.warmup):
         one_pass_device()
     n0, g0 = lib.mkd_launch_count(), sampler.graph_launches
     with ClockSampler(local) as clk:
-        ms = timed(one_pass_device, args.steps)
+        ms, last = timed(one_pass_device, args.steps)
     launches = (lib.mkd_launch_count() - n0) + (sampler.graph_launches - g0)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"images" if args.decode else "latents": last})
     for _ in range(2):
         one_pass_e2e()
-    ms_e2e = timed(one_pass_e2e, args.steps)
+    ms_e2e, _ = timed(one_pass_e2e, args.steps)
 
     ips = Bg * args.steps / (ms / 1e3)
     ips_e2e = Bg * args.steps / (ms_e2e / 1e3)

@@ -19,12 +19,14 @@ PARAMS = dict(model_channels=32, num_heads=2, context_dim=32)
 BG, H, S = 4, 8, 4
 
 
-def _setup_model():
+def _setup_model(patch=setattr):
+    """patch: plain setattr in a spawned worker; monkeypatch.setattr in the pytest process, where the fakes must not
+    outlive the test (later GPU tests would run them instead of the kernels)"""
     import fake_ops
     from makeupdiffuse_b200 import B200ControlLDM, B200DDIMSampler, ops
     from makeupdiffuse_b200.synth import synthetic_state_dict
     for name in fake_ops.ALL:
-        setattr(ops, name, getattr(fake_ops, name))
+        patch(ops, name, getattr(fake_ops, name))
     m = B200ControlLDM(PARAMS, PARAMS, dtype=torch.float32, device="cpu")
     m.load_state_dict(synthetic_state_dict(m, 0, device="cpu"))
     return B200DDIMSampler(m)
@@ -57,12 +59,12 @@ def test_shard_bounds():
     assert shard_bounds(5, 0, 1) == (0, 5)
 
 
-def test_two_rank_gloo_equals_single_process(tmp_path):
+def test_two_rank_gloo_equals_single_process(tmp_path, monkeypatch):
     port = 29500 + os.getpid() % 2000
     mp.spawn(_worker, args=(2, port, str(tmp_path)), nprocs=2, join=True)
     r0, r1 = torch.load(tmp_path / "r0.pt"), torch.load(tmp_path / "r1.pt")
     assert torch.equal(r0, r1) and r0.shape == (BG, 4, H, H)
-    s = _setup_model()
+    s = _setup_model(monkeypatch.setattr)
     d = _data()
     cond = {"c_crossattn": [d["ctx"]], "c_concat": [d["hint"]]}
     with torch.no_grad():
