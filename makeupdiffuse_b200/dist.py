@@ -10,6 +10,9 @@ only data-path collective is ONE all-gather of the final latents over NVLink 5 /
   other rank); the last DDIM update kernel stores its x_0 slice into ALL ranks' buffers itself
   (``mkd_ddim_update_peers``: plain stores to peer addresses over NVLink), and a signal barrier between the ranks
   replaces the collective launch.  Same bits as the NCCL path (tests/test_sharding.py, 2 GPUs).
+
+``sample_sharded`` runs the DDIM sampling loop this way; ``encode_sharded`` the DDIM inversion (x_0 -> x_t) of a
+dataset's latents, whose last inversion step writes into the gather buffer the same way.
 """
 from __future__ import annotations
 
@@ -39,6 +42,34 @@ def _symmetric_gather_buffer(shape, device, group):
     return hit
 
 
+def _gather_begin(batch_global, lo, hi, shape, device, world, group, fused_gather):
+    """the [batch_global, *shape] fp32 gather buffer, this rank's slice [lo, hi) of it, and for the fused gather the
+    rendezvous handle and the device pointers of that slice inside every rank's buffer.  The loop's last update writes
+    its result into the slice (``out=``) or into every rank's copy of it (``peer_ptrs=``)."""
+    if world > 1 and batch_global % world:
+        raise ValueError("sharded runs need batch_global % world == 0")
+    fused = bool(fused_gather) and world > 1
+    hdl = peer_ptrs = None
+    if fused:
+        gathered, hdl = _symmetric_gather_buffer((batch_global, *shape), device, group)
+        off = lo * int(np.prod(shape)) * 4
+        peer_ptrs = [int(p) + off for p in hdl.buffer_ptrs]  # this rank's slice inside every rank's buffer
+        hdl.barrier()  # nobody still reads the previous result out of the buffers we are about to overwrite
+    else:
+        gathered = torch.empty(batch_global, *shape, dtype=torch.float32, device=device)
+    return gathered, gathered[lo:hi], hdl, peer_ptrs
+
+
+def _gather_end(gathered, mine, hdl, world, group):
+    """completes the gather once the last update of every rank has been enqueued; returns the whole batch"""
+    if hdl is not None:
+        hdl.barrier()  # every rank's final update kernel has stored its slice everywhere
+        return gathered.clone()  # the symmetric buffer is reused by the next call
+    if world > 1:
+        dist.all_gather_into_tensor(gathered, mine, group=group)  # in place: input is the rank's own slice
+    return gathered
+
+
 def sample_sharded(sampler, S, batch_global, shape, cond_local, x_T_local, rank=0, world=1, group=None,
                    fused_gather=False, **kw):
     """DDIM-sample this rank's chunk and all-gather the final latents.
@@ -47,19 +78,8 @@ def sample_sharded(sampler, S, batch_global, shape, cond_local, x_T_local, rank=
     Requires equal chunk sizes when world > 1."""
     lo, hi = shard_bounds(batch_global, rank, world)
     b = hi - lo
-    C, H, W = shape
-    if world > 1 and batch_global % world:
-        raise ValueError("sample_sharded needs batch_global % world == 0")
-    fused = bool(fused_gather) and world > 1
-    hdl = peer_ptrs = None
-    if fused:
-        gathered, hdl = _symmetric_gather_buffer((batch_global, C, H, W), x_T_local.device, group)
-        off = lo * C * H * W * 4
-        peer_ptrs = [int(p) + off for p in hdl.buffer_ptrs]  # this rank's slice inside every rank's buffer
-        hdl.barrier()  # nobody still reads the previous result out of the buffers we are about to overwrite
-    else:
-        gathered = torch.empty(batch_global, C, H, W, dtype=torch.float32, device=x_T_local.device)
-    mine = gathered[lo:hi]
+    gathered, mine, hdl, peer_ptrs = _gather_begin(batch_global, lo, hi, tuple(shape), x_T_local.device, world, group,
+                                                   fused_gather)
     sampler.make_schedule(ddim_num_steps=S, ddim_eta=kw.pop("eta", 0.0), verbose=False)
     steps = np.flip(sampler.ddim_timesteps)
     own = hasattr(sampler, "begin_loop")
@@ -74,9 +94,19 @@ def sample_sharded(sampler, S, batch_global, shape, cond_local, x_T_local, rank=
             kw["t_value"] = int(step)
         x, _ = sampler.denoising_step(x, cond_local, ts, index=len(steps) - i - 1, out=mine if last else None,
                                       peer_ptrs=peer_ptrs if last else None, **kw)
-    if fused:
-        hdl.barrier()  # every rank's final update kernel has stored its slice everywhere
-        return gathered.clone()  # the symmetric buffer is reused by the next call
-    if world > 1:
-        dist.all_gather_into_tensor(gathered, mine, group=group)  # in place: input is the rank's own slice
-    return gathered
+    return _gather_end(gathered, mine, hdl, world, group)
+
+
+def encode_sharded(sampler, t_enc, batch_global, x0_local, cond_local, rank=0, world=1, group=None, fused_gather=False,
+                   **kw):
+    """DDIM-invert this rank's chunk (B200DDIMSampler.encode on the schedule already set) and all-gather the x_t.
+
+    x0_local / cond_local hold this rank's rows only; kw goes to encode (guidance, use_original_steps, callback).
+    Returns the [batch_global, C, H, W] inverted latents on every rank.  Requires equal chunk sizes when world > 1."""
+    if t_enc < 1:
+        raise ValueError("encode_sharded needs t_enc >= 1: the last inversion step writes the gathered result")
+    lo, hi = shard_bounds(batch_global, rank, world)
+    gathered, mine, hdl, peer_ptrs = _gather_begin(batch_global, lo, hi, tuple(x0_local.shape[1:]), x0_local.device, world,
+                                                   group, fused_gather)
+    sampler.encode(x0_local, cond_local, t_enc, out=mine, peer_ptrs=peer_ptrs, **kw)
+    return _gather_end(gathered, mine, hdl, world, group)

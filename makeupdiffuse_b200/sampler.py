@@ -1,7 +1,7 @@
 """``B200DDIMSampler``: drop-in for ``MKDDIMSampler`` (diffmk/cddim.py:5-100) and the upstream ``DDIMSampler`` it
 extends — same constructor, same ``make_schedule`` / ``sample`` / ``ddim_sampling`` / ``p_sample_ddim`` /
-``denoising_step`` / ``reconstruct`` / ``decode`` / ``stochastic_encode`` signatures and return values
-(SURVEY.md §8(b) level B1).
+``denoising_step`` / ``reconstruct`` / ``decode`` / ``stochastic_encode`` / ``encode`` (DDIM inversion) signatures and
+return values (SURVEY.md §8(b) level B1).
 
 Per step it runs ``model.apply_model`` (one CUDA-graph replay of the fused UNet+ControlNet kernels when
 ``use_cuda_graph`` is on) followed by ONE fused kernel for the whole x_t -> x_{t-1} update including the
@@ -159,6 +159,13 @@ class B200DDIMSampler:
         with torch.no_grad():
             return self.reconstruct(x_latent, cond, t_start, **kw)
 
+    def _cfg_cond(self, c, uc):
+        """[uncond; cond] for the doubled batch; step-invariant, so built once per loop, not once per step"""
+        cc = self._cfg_cache
+        if cc is None or cc[0] is not c or cc[1] is not uc:
+            cc = self._cfg_cache = (c, uc, _cat_uncond_first(uc, c))
+        return cc[2]
+
     # ---- the model call, optionally as a CUDA-graph replay -------------------------------------------------------
     def _eps(self, x, t, c, t_value=None):
         """model.apply_model(x, t, c); with use_cuda_graph the ~10^3 kernel launches of one UNet+ControlNet step are
@@ -236,10 +243,7 @@ class B200DDIMSampler:
         if not cfg:
             e = self._eps(x, t, c, t_value)
         else:
-            cc = self._cfg_cache  # the doubled cond is step-invariant: build it once, not 50 times
-            if cc is None or cc[0] is not c or cc[1] is not unconditional_conditioning:
-                cc = self._cfg_cache = (c, unconditional_conditioning, _cat_uncond_first(unconditional_conditioning, c))
-            e = self._eps(torch.cat([x] * 2), torch.cat([t] * 2), cc[2], t_value)
+            e = self._eps(torch.cat([x] * 2), torch.cat([t] * 2), self._cfg_cond(c, unconditional_conditioning), t_value)
         if use_original_steps:
             if self._coef_orig is None:
                 # cddim.py:54 reads the sigma table off the MODEL; without that attribute the reference raises
@@ -282,3 +286,64 @@ class B200DDIMSampler:
             if callback:
                 callback(i)
         return x
+
+    # ---- DDIM inversion x_0 -> x_t (upstream DDIMSampler.encode; the loop that produces reconstruct's x_latent) --------
+    @staticmethod
+    def _encode_coefficients(alphas_next, alphas):
+        """per step (c_x, c_e) with x_next = c_x * x + c_e * eps: upstream's expressions on upstream's operands (fp32
+        alphas_next on the model's device; fp64 alphas on the CPU for the DDIM schedule, the fp32 device table with
+        use_original_steps), each rounded to fp32 once as the multiply with the fp32 latent does.  They are evaluated where
+        upstream evaluates them, as 0-dim tensors on the same devices: c_e subtracts two nearly equal square roots, and the
+        same expressions evaluated on the CPU instead gave another fp32 update on a B200 (one ulp, step 6 of S = 20 and 50)."""
+        cx, ce = [], []
+        for an, a in zip(alphas_next, alphas):
+            cx.append((an / a).sqrt().float())
+            ce.append((an.sqrt() * ((1 / an - 1).sqrt() - (1 / a - 1).sqrt())).float())
+        return list(zip(torch.stack(cx).tolist(), torch.stack(ce).tolist())) if cx else []
+
+    @torch.no_grad()
+    def encode(self, x0, c, t_enc, use_original_steps=False, return_intermediates=None, unconditional_guidance_scale=1.0,
+               unconditional_conditioning=None, callback=None, out=None, peer_ptrs=None):
+        """Deterministic DDIM inversion: t_enc steps from the clean latent x0 towards noise, on the schedule set by the last
+        make_schedule.  Returns (x_t, {"x_encoded", "intermediate_steps"[, "intermediates"]}) like upstream; draws no noise.
+        ``out`` / ``peer_ptrs`` (extensions, optional): as in denoising_step, for the LAST step only."""
+        num_reference_steps = self.ddpm_num_timesteps if use_original_steps else self.ddim_timesteps.shape[0]
+        assert t_enc <= num_reference_steps
+        if use_original_steps:
+            alphas_next, alphas = self.alphas_cumprod[:t_enc], self.alphas_cumprod_prev[:t_enc]
+        else:
+            alphas_next, alphas = self.ddim_alphas[:t_enc], torch.tensor(self.ddim_alphas_prev[:t_enc])
+        coef = self._encode_coefficients(alphas_next, alphas)  # once per call, before the loop
+        cfg = unconditional_guidance_scale != 1.0
+        if cfg:
+            assert unconditional_conditioning is not None
+        self.begin_loop(range(t_enc))
+        x_next = x0
+        intermediates, inter_steps = [], []
+        for i in range(t_enc):
+            x = x_next.float().contiguous()
+            t = torch.full((x.shape[0],), i, device=self.model.device, dtype=torch.long)  # the loop index, as upstream
+            if not cfg:
+                e = self._eps(x, t, c, t_value=i)
+            else:
+                e = self._eps(torch.cat([x] * 2), torch.cat([t] * 2), self._cfg_cond(c, unconditional_conditioning), t_value=i)
+            last = i == t_enc - 1
+            x_next = out if (last and out is not None) else torch.empty_like(x)
+            c_x, c_e = coef[i]
+            # the sampling kernel with sqrt(1-a_t) = 0, sqrt(a_t) = 1 computes fl(c_x * fl(fl(x - 0*e) / 1)) + fl(c_e * e):
+            # for finite values that is upstream's fl(c_x * x) + fl(c_e * e), so the inversion needs no kernel of its own
+            ops.ddim_update(x, e.contiguous(), x_next, sqrt_one_minus_at=0.0, sqrt_at=1.0, sqrt_a_prev=c_x, dir_coef=c_e,
+                            cfg_scale=float(unconditional_guidance_scale) if cfg else None,
+                            peer_ptrs=peer_ptrs if last else None)
+            if return_intermediates and i % (t_enc // return_intermediates) == 0 and i < t_enc - 1:
+                intermediates.append(x_next)
+                inter_steps.append(i)
+            elif return_intermediates and i >= t_enc - 2:
+                intermediates.append(x_next)
+                inter_steps.append(i)
+            if callback:
+                callback(i)
+        res = {"x_encoded": x_next, "intermediate_steps": inter_steps}
+        if return_intermediates:
+            res["intermediates"] = intermediates
+        return x_next, res
