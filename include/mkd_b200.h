@@ -31,7 +31,7 @@
 extern "C" {
 #endif
 
-#define MKD_ABI_VERSION 10
+#define MKD_ABI_VERSION 11
 
 typedef void* mkd_stream_t; /* cudaStream_t */
 
@@ -69,6 +69,36 @@ int mkd_ddim_update_peers(const float* x, const float* eps, int cfg, float cfg_s
                           float sqrt_one_minus_at, float sqrt_at, float sqrt_a_prev, float dir_coef, float sigma_t,
                           float temperature, float* const* x_prev_peers, int n_peers, float* pred_x0, int64_t n,
                           mkd_stream_t stream);
+
+/* ---- PLMS x_t -> x_{t-1} update (ABI v11) -------------------------------------------------------------------
+ * replaces upstream ldm/models/diffusion/plms.py p_sample_plms after its model call(s): get_model_output's CFG combine,
+ * the pseudo-improved-Euler / Adams-Bashforth combination of the current and up to three earlier eps, and
+ * get_x_prev_and_pred_x0 (the DDIM update at sigma == 0, which PLMS requires: eta must be 0).
+ *   e       = cfg ? eps[0:n] + cfg_scale * (eps[n:2n] - eps[0:n]) : eps[0:n]       ([uncond; cond] order)
+ *   e_store = e                                                                    (skipped when e_store is NULL)
+ *   e'      = mode 0: e                                      (plain DDIM update, e.g. the first half of step 0)
+ *             mode 1: (h1 + e) / 2                           (step 0: h1 = e_t, e = e_next)
+ *             mode 2: (3 e - h1) / 2
+ *             mode 3: (23 e - 16 h1 + 5 h2) / 12
+ *             mode 4: (55 e - 59 h1 + 37 h2 - 9 h3) / 24     (h1 = o[-1] the newest earlier e_t, h3 = o[-3] the oldest)
+ *   pred_x0 = (x - sqrt_one_minus_at * e') / sqrt_at
+ *   x_prev  = sqrt_a_prev * pred_x0 + dir_coef * e'
+ * Every product/sum is rounded separately in upstream's order (no FMA contraction); the divisions by 2, 12 and 24 are
+ * products with the fp32 reciprocals, which is how torch on CUDA evaluates a tensor divided by a Python scalar, so the
+ * result is bit-identical to upstream's fp32 torch arithmetic on the GPU.  h1..h3 are read only as the mode needs them.
+ * Aliasing: x_prev may alias x, and e_store may alias h3 (the ring slot of the oldest eps is overwritten by the newest);
+ * no other pointers may overlap.  pred_x0 may be NULL. */
+int mkd_plms_update(const float* x, const float* eps, int cfg, float cfg_scale, float* e_store, int mode, const float* h1,
+                    const float* h2, const float* h3, float sqrt_one_minus_at, float sqrt_at, float sqrt_a_prev,
+                    float dir_coef, float* x_prev, float* pred_x0, int64_t n, mkd_stream_t stream);
+
+/* The same update with x_prev written to n_peers (1..8) destinations, as mkd_ddim_update_peers: the last step of a
+ * batch-sharded PLMS run stores its slice of the all-gathered result into every rank's gather buffer.  Values are
+ * bit-identical to mkd_plms_update. */
+int mkd_plms_update_peers(const float* x, const float* eps, int cfg, float cfg_scale, float* e_store, int mode,
+                          const float* h1, const float* h2, const float* h3, float sqrt_one_minus_at, float sqrt_at,
+                          float sqrt_a_prev, float dir_coef, float* const* x_prev_peers, int n_peers, float* pred_x0,
+                          int64_t n, mkd_stream_t stream);
 
 /* ---- layout / small elementwise ---------------------------------------------------------------------------
  * NCHW fp32 (the reference boundary layout, makeup_diffuse.py:152) <-> NHWC working layout. */

@@ -141,6 +141,91 @@ extern "C" int mkd_ddim_update(const float* x, const float* eps, int cfg, float 
 }
 
 // ---------------------------------------------------------------------------------------------------------
+// PLMS update (upstream ldm/models/diffusion/plms.py p_sample_plms): the CFG combine, the store of e_t into the
+// sampler's history ring, the Adams-Bashforth combination e' of up to four eps and the DDIM update on e', in one pass.
+// e_store / h1..h3 / x / x_prev carry no __restrict__: the header allows e_store == h3 and x_prev == x, and each thread
+// reads every input element before it stores its own.  Torch on CUDA evaluates `t / k` with a CPU-scalar k as
+// t * fl(1 / k) (ATen div_true_kernel_cuda), so the divisors 2, 12 and 24 are applied as products with those reciprocals.
+// ---------------------------------------------------------------------------------------------------------
+template <int NP>
+__global__ void plms_update_kernel(const float* x, const float* __restrict__ eps, int cfg, float cfg_scale, float* e_store,
+                                   int mode, const float* h1, const float* h2, const float* h3, float s1m, float sqrt_at,
+                                   float sqrt_ap, float dirc, PeerPtrs out, float* pred_x0, int64_t n) {
+  pdl_wait();
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+    float e = eps[i];
+    if (cfg) e = __fadd_rn(e, __fmul_rn(cfg_scale, __fsub_rn(eps[n + i], e)));  // e_u + s * (e_c - e_u)   plms.py get_model_output
+    float ep = e;
+    if (mode == 1) {  // pseudo improved Euler: (e_t + e_next) / 2, e_t from the history
+      ep = __fmul_rn(__fadd_rn(h1[i], e), 0.5f);
+    } else if (mode == 2) {  // (3 e_t - o[-1]) / 2
+      ep = __fmul_rn(__fsub_rn(__fmul_rn(3.0f, e), h1[i]), 0.5f);
+    } else if (mode == 3) {  // (23 e_t - 16 o[-1] + 5 o[-2]) / 12
+      ep = __fmul_rn(__fadd_rn(__fsub_rn(__fmul_rn(23.0f, e), __fmul_rn(16.0f, h1[i])), __fmul_rn(5.0f, h2[i])), 1.0f / 12.0f);
+    } else if (mode == 4) {  // (55 e_t - 59 o[-1] + 37 o[-2] - 9 o[-3]) / 24
+      float s = __fsub_rn(__fmul_rn(55.0f, e), __fmul_rn(59.0f, h1[i]));
+      s = __fsub_rn(__fadd_rn(s, __fmul_rn(37.0f, h2[i])), __fmul_rn(9.0f, h3[i]));
+      ep = __fmul_rn(s, 1.0f / 24.0f);
+    }
+    float p0 = __fdiv_rn(__fsub_rn(x[i], __fmul_rn(s1m, ep)), sqrt_at);  // get_x_prev_and_pred_x0 (= cddim.py:63,74,78)
+    float xp = __fadd_rn(__fmul_rn(sqrt_ap, p0), __fmul_rn(dirc, ep));
+    if (e_store) e_store[i] = e;
+    if (pred_x0) pred_x0[i] = p0;
+#pragma unroll
+    for (int r = 0; r < NP; ++r) out.p[r][i] = xp;
+  }
+}
+
+static int plms_launch(const float* x, const float* eps, int cfg, float cfg_scale, float* e_store, int mode, const float* h1,
+                       const float* h2, const float* h3, float s1m, float sqrt_at, float sqrt_ap, float dirc,
+                       const PeerPtrs& pp, int n_peers, float* pred_x0, int64_t n, mkd_stream_t stream, const char* who) {
+  MKD_REQUIRE(x && eps && n >= 0, MKD_E_INVALID, "%s: null pointer or negative n", who);
+  MKD_REQUIRE(mode >= 0 && mode <= 4, MKD_E_INVALID, "%s: mode=%d must be 0..4", who, mode);
+  MKD_REQUIRE((mode < 1 || h1) && (mode < 3 || h2) && (mode < 4 || h3), MKD_E_INVALID,
+              "%s: mode %d needs %d history pointer(s)", who, mode, mode <= 2 ? 1 : mode - 1);
+  for (int r = 0; r < n_peers; ++r) MKD_REQUIRE(pp.p[r] != nullptr, MKD_E_INVALID, "%s: null x_prev pointer %d", who, r);
+  if (n == 0) return MKD_OK;
+  int threads = 256;
+  int blocks = (int)((n + threads - 1) / threads);
+  if (blocks > 148 * 8) blocks = 148 * 8;
+  cudaStream_t st = (cudaStream_t)stream;
+#define MKD_PLMS_CASE(NP)                                                                                               \
+  case NP:                                                                                                              \
+    MKD_LAUNCH_OK(launch_pdl(plms_update_kernel<NP>, dim3(blocks), dim3(threads), 0, st, x, eps, cfg, cfg_scale, e_store, \
+                             mode, h1, h2, h3, s1m, sqrt_at, sqrt_ap, dirc, pp, pred_x0, n));                           \
+    break;
+  switch (n_peers) {
+    MKD_PLMS_CASE(1) MKD_PLMS_CASE(2) MKD_PLMS_CASE(3) MKD_PLMS_CASE(4)
+    MKD_PLMS_CASE(5) MKD_PLMS_CASE(6) MKD_PLMS_CASE(7) MKD_PLMS_CASE(8)
+  }
+#undef MKD_PLMS_CASE
+  MKD_CHECK_LAUNCH();
+  return MKD_OK;
+}
+
+extern "C" int mkd_plms_update(const float* x, const float* eps, int cfg, float cfg_scale, float* e_store, int mode,
+                               const float* h1, const float* h2, const float* h3, float sqrt_one_minus_at, float sqrt_at,
+                               float sqrt_a_prev, float dir_coef, float* x_prev, float* pred_x0, int64_t n,
+                               mkd_stream_t stream) {
+  PeerPtrs pp = {};
+  pp.p[0] = x_prev;
+  return plms_launch(x, eps, cfg, cfg_scale, e_store, mode, h1, h2, h3, sqrt_one_minus_at, sqrt_at, sqrt_a_prev, dir_coef,
+                     pp, 1, pred_x0, n, stream, "plms_update");
+}
+
+extern "C" int mkd_plms_update_peers(const float* x, const float* eps, int cfg, float cfg_scale, float* e_store, int mode,
+                                     const float* h1, const float* h2, const float* h3, float sqrt_one_minus_at,
+                                     float sqrt_at, float sqrt_a_prev, float dir_coef, float* const* x_prev_peers,
+                                     int n_peers, float* pred_x0, int64_t n, mkd_stream_t stream) {
+  MKD_REQUIRE(x_prev_peers, MKD_E_INVALID, "plms_update_peers: null peer array");
+  MKD_REQUIRE(n_peers >= 1 && n_peers <= 8, MKD_E_INVALID, "plms_update_peers: n_peers=%d must be 1..8 (one box)", n_peers);
+  PeerPtrs pp = {};
+  for (int r = 0; r < n_peers; ++r) pp.p[r] = x_prev_peers[r];  // host array of device pointers
+  return plms_launch(x, eps, cfg, cfg_scale, e_store, mode, h1, h2, h3, sqrt_one_minus_at, sqrt_at, sqrt_a_prev, dir_coef,
+                     pp, n_peers, pred_x0, n, stream, "plms_update_peers");
+}
+
+// ---------------------------------------------------------------------------------------------------------
 // NCHW fp32 <-> NHWC T through a 32x32 smem transpose tile (coalesced on both sides).
 // ---------------------------------------------------------------------------------------------------------
 template <typename T>

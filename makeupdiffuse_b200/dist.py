@@ -12,7 +12,8 @@ only data-path collective is ONE all-gather of the final latents over NVLink 5 /
   replaces the collective launch.  Same bits as the NCCL path (tests/test_sharding.py, 2 GPUs).
 
 ``sample_sharded`` runs the DDIM sampling loop this way; ``encode_sharded`` the DDIM inversion (x_0 -> x_t) of a
-dataset's latents, whose last inversion step writes into the gather buffer the same way.
+dataset's latents, whose last inversion step writes into the gather buffer the same way; ``sample_plms_sharded`` the PLMS
+sampling loop (B200PLMSSampler), whose last update kernel (``mkd_plms_update[_peers]``) does the same.
 """
 from __future__ import annotations
 
@@ -94,6 +95,20 @@ def sample_sharded(sampler, S, batch_global, shape, cond_local, x_T_local, rank=
             kw["t_value"] = int(step)
         x, _ = sampler.denoising_step(x, cond_local, ts, index=len(steps) - i - 1, out=mine if last else None,
                                       peer_ptrs=peer_ptrs if last else None, **kw)
+    return _gather_end(gathered, mine, hdl, world, group)
+
+
+def sample_plms_sharded(sampler, S, batch_global, shape, cond_local, x_T_local, rank=0, world=1, group=None,
+                        fused_gather=False, **kw):
+    """PLMS-sample this rank's chunk (B200PLMSSampler.sample) and all-gather the final latents.
+
+    Arguments as sample_sharded; kw goes to sample (eta, guidance, callbacks).  Returns the [batch_global, C, H, W] latents
+    on every rank.  Requires equal chunk sizes when world > 1."""
+    lo, hi = shard_bounds(batch_global, rank, world)
+    gathered, mine, hdl, peer_ptrs = _gather_begin(batch_global, lo, hi, tuple(shape), x_T_local.device, world, group,
+                                                   fused_gather)
+    kw.setdefault("verbose", False)
+    sampler.sample(S, hi - lo, tuple(shape), cond_local, x_T=x_T_local, out=mine, peer_ptrs=peer_ptrs, **kw)
     return _gather_end(gathered, mine, hdl, world, group)
 
 

@@ -89,6 +89,37 @@ def ddim_update(x, eps, x_prev, *, sqrt_one_minus_at, sqrt_at, sqrt_a_prev, dir_
             "ddim_update")
 
 
+PLMS_HISTORY = (0, 1, 1, 2, 3)  # earlier eps each mode of mkd_plms_update reads
+
+
+def plms_update(x, eps, x_prev, *, mode, history=(), e_store=None, sqrt_one_minus_at, sqrt_at, sqrt_a_prev, dir_coef,
+                pred_x0=None, cfg_scale=None, peer_ptrs=None):
+    """One PLMS update (upstream plms.py p_sample_plms after its model call): eps holds n values, or 2n ([uncond; cond]) when
+    cfg_scale is given; the combined e_t goes to e_store when given.  history: the earlier eps the mode combines, newest
+    first (upstream's old_eps[-1], old_eps[-2], old_eps[-3]); mode 1 averages with history[0] (the pseudo improved Euler
+    step), modes 2 / 3 / 4 are the Adams-Bashforth orders, mode 0 is the plain DDIM update."""
+    n = x.numel()
+    if not 0 <= mode <= 4 or len(history) != PLMS_HISTORY[mode]:
+        raise ValueError(f"plms_update mode {mode} takes {PLMS_HISTORY[mode] if 0 <= mode <= 4 else '?'} history tensors")
+    for t in (x, eps, x_prev, e_store, pred_x0, *history):
+        if t is not None and (t.dtype != torch.float32 or not t.is_contiguous() or not t.is_cuda):
+            raise ValueError("plms_update works on contiguous fp32 CUDA latents")
+    for t in (x_prev, e_store, pred_x0, *history):
+        if t is not None and t.numel() != n:
+            raise ValueError("plms_update: every latent-sized tensor must hold x.numel() values")
+    cfg = cfg_scale is not None
+    if eps.numel() != (2 * n if cfg else n):
+        raise ValueError("eps has the wrong number of elements")
+    h = [_p(t) for t in history] + [None] * (3 - len(history))
+    head = (x.data_ptr(), eps.data_ptr(), int(cfg), float(cfg_scale or 0.0), _p(e_store), int(mode), *h,
+            float(sqrt_one_minus_at), float(sqrt_at), float(sqrt_a_prev), float(dir_coef))
+    if peer_ptrs is not None:  # x_prev goes to every rank's gather buffer (mkd_plms_update_peers); x_prev = own slice
+        arr = (C.c_void_p * len(peer_ptrs))(*[int(p) for p in peer_ptrs])
+        L.check(L.load().mkd_plms_update_peers(*head, arr, len(peer_ptrs), _p(pred_x0), n, _stream()), "plms_update_peers")
+        return
+    L.check(L.load().mkd_plms_update(*head, x_prev.data_ptr(), _p(pred_x0), n, _stream()), "plms_update")
+
+
 @_timed("nchw_to_nhwc", lambda s, d: _nb(s, d))
 def nchw_to_nhwc(src, dst2d):
     N, Cc, H, W = src.shape

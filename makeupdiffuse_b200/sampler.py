@@ -8,6 +8,9 @@ Per step it runs ``model.apply_model`` (one CUDA-graph replay of the fused UNet+
 classifier-free-guidance combine (cddim.py:39-40, 56-78), instead of ~12 elementwise launches + 4 ``torch.full``.
 The RNG stream is consumed exactly like the reference: one ``randn(x.shape)`` per step even when sigma == 0
 (cddim.py:75).  Unlike upstream nothing is force-moved to "cuda": buffers follow ``model.device``.
+
+``B200PLMSSampler`` (below) is the drop-in for upstream ``PLMSSampler`` on the same machinery, with its own fused update
+kernel (mkd_plms_update).
 """
 from __future__ import annotations
 
@@ -75,10 +78,11 @@ class B200DDIMSampler:
         self._coef_orig = None
 
     @staticmethod
-    def _coefficients(A, AP, S1, SG):
+    def _coefficients(A, AP, S1, SG, device=None):
         """per index: (sqrt(1-a_t), sqrt(a_t), sqrt(a_prev), sqrt(1 - a_prev - sigma^2), sigma) as fp32 values
-        (cddim.py:56-59 builds fp32 tensors with torch.full; :63,74,78 take fp32 sqrt)"""
-        f = lambda v: torch.as_tensor(np.asarray(v.cpu() if torch.is_tensor(v) else v), dtype=torch.float32)  # noqa: E731
+        (cddim.py:56-59 builds fp32 tensors with torch.full; :63,74,78 take fp32 sqrt), evaluated on ``device`` (the CPU
+        by default)"""
+        f = lambda v: torch.as_tensor(np.asarray(v.cpu() if torch.is_tensor(v) else v), dtype=torch.float32, device=device)  # noqa: E731
         a, ap, s1, sg = f(A), f(AP), f(S1), f(SG)
         return torch.stack([s1, a.sqrt(), ap.sqrt(), (1.0 - ap - sg ** 2).sqrt(), sg], 1).tolist()
 
@@ -347,3 +351,131 @@ class B200DDIMSampler:
         if return_intermediates:
             res["intermediates"] = intermediates
         return x_next, res
+
+
+class B200PLMSSampler(B200DDIMSampler):
+    """Drop-in for upstream ``ldm.models.diffusion.plms.PLMSSampler``: DDIM's schedule (eta must be 0), timesteps and
+    coefficients, with the eps of each step replaced by a pseudo-linear multistep combination of the current and up to
+    three earlier eps.  A run of S steps makes S + 1 model evaluations (step 0 evaluates twice) and draws S + 1
+    ``randn(x.shape)`` like upstream.  Per evaluation: one graph-replayed UNet+ControlNet call, then one fused kernel
+    (mkd_plms_update) for the CFG combine, the store of e_t into a ring of three device buffers, the combination and the
+    DDIM update.  One deliberate superset: the guided call accepts this model's dict-of-lists cond (upstream's
+    ``torch.cat([uc, c])`` takes bare tensors only)."""
+
+    def make_schedule(self, ddim_num_steps, ddim_discretize="uniform", ddim_eta=0.0, verbose=True):
+        if ddim_eta != 0:
+            raise ValueError("ddim_eta must be 0 for PLMS")
+        super().make_schedule(ddim_num_steps, ddim_discretize=ddim_discretize, ddim_eta=ddim_eta, verbose=verbose)
+        # the square roots on the model's device, where upstream takes them: torch's fp32 sqrt on the CPU is one ulp off the
+        # correctly rounded CUDA result at a few entries of the 50-step schedule (sqrt(a_t) at indices 6 and 44)
+        self._coef_ddim = self._coefficients(self.ddim_alphas, self.ddim_alphas_prev, self.ddim_sqrt_one_minus_alphas,
+                                             self.ddim_sigmas, device=self.model.device)
+
+    def sample(self, S, batch_size, shape, conditioning=None, callback=None, normals_sequence=None, img_callback=None,
+               quantize_x0=False, eta=0.0, mask=None, x0=None, temperature=1.0, noise_dropout=0.0, score_corrector=None,
+               corrector_kwargs=None, verbose=True, x_T=None, log_every_t=100, unconditional_guidance_scale=1.0,
+               unconditional_conditioning=None, dynamic_threshold=None, out=None, peer_ptrs=None, **kwargs):
+        """``out`` / ``peer_ptrs`` (extensions, optional): as in denoising_step, for the LAST update only"""
+        self.make_schedule(ddim_num_steps=S, ddim_eta=eta, verbose=verbose)
+        C, H, W = shape
+        return self.plms_sampling(conditioning, (batch_size, C, H, W), callback=callback, img_callback=img_callback,
+                                  quantize_denoised=quantize_x0, mask=mask, x0=x0, ddim_use_original_steps=False,
+                                  noise_dropout=noise_dropout, temperature=temperature, score_corrector=score_corrector,
+                                  corrector_kwargs=corrector_kwargs, x_T=x_T, log_every_t=log_every_t,
+                                  unconditional_guidance_scale=unconditional_guidance_scale,
+                                  unconditional_conditioning=unconditional_conditioning,
+                                  dynamic_threshold=dynamic_threshold, out=out, peer_ptrs=peer_ptrs)
+
+    @torch.no_grad()
+    def plms_sampling(self, cond, shape, x_T=None, ddim_use_original_steps=False, callback=None, timesteps=None,
+                      quantize_denoised=False, mask=None, x0=None, img_callback=None, log_every_t=100, temperature=1.0,
+                      noise_dropout=0.0, score_corrector=None, corrector_kwargs=None, unconditional_guidance_scale=1.0,
+                      unconditional_conditioning=None, dynamic_threshold=None, out=None, peer_ptrs=None):
+        if ddim_use_original_steps or timesteps is not None:
+            raise NotImplementedError("the B200 PLMS loop runs the DDIM schedule set by make_schedule")
+        dev = self.model.device
+        b = shape[0]
+        img = torch.randn(shape, device=dev) if x_T is None else x_T
+        time_range = np.flip(self.ddim_timesteps)
+        total = time_range.shape[0]
+        self.begin_loop(time_range)
+        # the eps history: three device buffers reused round-robin, so a step writes no tensor of its own for it; the slot
+        # a step writes is the one of the oldest eps, which AB4 reads in the same kernel
+        ring = torch.empty((3, *shape), device=dev, dtype=torch.float32)
+        inter = {"x_inter": [img], "pred_x0": [img]}
+        old_eps = []
+        for i, step in enumerate(time_range):
+            index = total - i - 1
+            step_next = int(time_range[min(i + 1, total - 1)])
+            ts = torch.full((b,), int(step), device=dev, dtype=torch.long)
+            ts_next = torch.full((b,), step_next, device=dev, dtype=torch.long)
+            if mask is not None:
+                img = self.model.q_sample(x0, ts) * mask + (1.0 - mask) * img
+            last = i == total - 1
+            img, pred_x0, e_t = self.p_sample_plms(
+                img, cond, ts, index=index, quantize_denoised=quantize_denoised, temperature=temperature,
+                noise_dropout=noise_dropout, score_corrector=score_corrector, corrector_kwargs=corrector_kwargs,
+                unconditional_guidance_scale=unconditional_guidance_scale,
+                unconditional_conditioning=unconditional_conditioning, old_eps=old_eps, t_next=ts_next,
+                dynamic_threshold=dynamic_threshold, e_t_out=ring[i % 3], t_value=int(step), t_next_value=step_next,
+                out=out if last else None, peer_ptrs=peer_ptrs if last else None)
+            old_eps.append(e_t)
+            if len(old_eps) >= 4:
+                old_eps.pop(0)
+            if callback:
+                callback(i)
+            if img_callback:
+                img_callback(pred_x0, i)
+            if index % log_every_t == 0 or index == total - 1:
+                inter["x_inter"].append(img)
+                inter["pred_x0"].append(pred_x0)
+        return img, inter
+
+    @torch.no_grad()
+    def p_sample_plms(self, x, c, t, index, repeat_noise=False, use_original_steps=False, quantize_denoised=False,
+                      temperature=1.0, noise_dropout=0.0, score_corrector=None, corrector_kwargs=None,
+                      unconditional_guidance_scale=1.0, unconditional_conditioning=None, old_eps=None, t_next=None,
+                      dynamic_threshold=None, e_t_out=None, t_value=None, t_next_value=None, out=None, peer_ptrs=None):
+        """upstream p_sample_plms: returns (x_prev, pred_x0, e_t).  With no earlier eps it evaluates the model a second
+        time, at ``t_next``, on the plain DDIM update of x (pseudo improved Euler).
+        Extensions (optional): ``e_t_out`` receives e_t (a fresh tensor otherwise); ``t_value`` / ``t_next_value`` are the
+        timesteps of ``t`` / ``t_next`` as host ints (see _eps); ``out`` / ``peer_ptrs`` as in denoising_step."""
+        m = self.model
+        if m.parameterization != "eps":
+            raise NotImplementedError("B200 path implements the yaml's parameterization: eps (yaml:50)")
+        if score_corrector is not None or quantize_denoised:
+            raise NotImplementedError("score_corrector / quantize_denoised are unused by the reference path")
+        if dynamic_threshold is not None or use_original_steps:
+            raise NotImplementedError()
+        old_eps = list(old_eps or [])[-3:]  # upstream's ">= 3" branch reads the newest three
+        x = x.float().contiguous()
+        cfg = not (unconditional_conditioning is None or unconditional_guidance_scale == 1.0)
+        cc = self._cfg_cond(c, unconditional_conditioning) if cfg else c
+        scale = float(unconditional_guidance_scale) if cfg else None
+        s1m, sq_at, sq_ap, dirc, _ = self._coef_ddim[index]  # sigma == 0: make_schedule insists on eta == 0
+        coef = dict(sqrt_one_minus_at=s1m, sqrt_at=sq_at, sqrt_a_prev=sq_ap, dir_coef=dirc)
+
+        def model_output(xx, tt, tv):
+            if not cfg:
+                return self._eps(xx, tt, c, tv).contiguous()
+            return self._eps(torch.cat([xx] * 2), torch.cat([tt] * 2), cc, tv).contiguous()
+
+        def draw():
+            # upstream draws the noise in every get_x_prev_and_pred_x0, and sigma is 0: keep the RNG stream in step
+            torch.randn((1, *x.shape[1:]) if repeat_noise else x.shape, device=x.device)
+
+        e_t = torch.empty_like(x) if e_t_out is None else e_t_out
+        x_prev, pred_x0 = (torch.empty_like(x) if out is None else out), torch.empty_like(x)
+        eps = model_output(x, t, t_value)
+        if not old_eps:
+            # e_t lands in its slot before the second evaluation overwrites the graph's output buffer
+            ops.plms_update(x, eps, pred_x0, mode=0, e_store=e_t, cfg_scale=scale, **coef)  # x_pred, in pred_x0's buffer
+            draw()
+            eps = model_output(pred_x0, t_next, t_next_value)
+            mode, history, store = 1, (e_t,), None
+        else:
+            mode, history, store = len(old_eps) + 1, tuple(reversed(old_eps)), e_t
+        ops.plms_update(x, eps, x_prev, mode=mode, history=history, e_store=store, cfg_scale=scale, pred_x0=pred_x0,
+                        peer_ptrs=peer_ptrs, **coef)
+        draw()
+        return x_prev, pred_x0, e_t
