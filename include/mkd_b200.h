@@ -31,7 +31,7 @@
 extern "C" {
 #endif
 
-#define MKD_ABI_VERSION 11
+#define MKD_ABI_VERSION 12
 
 typedef void* mkd_stream_t; /* cudaStream_t */
 
@@ -100,6 +100,32 @@ int mkd_plms_update_peers(const float* x, const float* eps, int cfg, float cfg_s
                           float sqrt_a_prev, float dir_coef, float* const* x_prev_peers, int n_peers, float* pred_x0,
                           int64_t n, mkd_stream_t stream);
 
+/* ---- DPM-Solver++ multistep update (ABI v12) ------------------------------------------------------------------
+ * replaces upstream ldm/models/diffusion/dpm_solver/dpm_solver.py after one model call (DPMSolver with predict_x0=True,
+ * method 'multistep', solver_type 'dpm_solver'): model_wrapper's classifier-free combine, data_prediction_fn at the
+ * evaluated time s = t_k, and multistep_dpm_solver_update from s to the next time t = t_{k+1} of order 1
+ * (dpm_solver_first_update) or 2 (multistep_dpm_solver_second_update).
+ *   e       = cfg ? eps[0:n] + cfg_scale * (eps[n:2n] - eps[0:n]) : eps[0:n]       ([uncond; cond] order)
+ *   m       = (x - sigma_s * e) / alpha_s                                          (the data prediction m_k)
+ *   m_store = m                                                                    (skipped when m_store is NULL)
+ *   order 1: x_prev = sigma_ratio * x - phi * m                      (sigma_ratio = sigma_t / sigma_s, phi = alpha_t * expm1(-h))
+ *   order 2: D      = inv_r0 * (m - m_prev)                          (m_prev = m_{k-1}, inv_r0 = 1 / r0)
+ *            x_prev = sigma_ratio * x - phi * m - half_phi * D       (phi = alpha_t * (exp(-h) - 1), half_phi = 0.5 * phi)
+ * The scalars are the caller's, evaluated with upstream's torch expressions on the device.  Every product, sum and the
+ * true division are rounded separately in upstream's order (no FMA contraction), so the result is bit-identical to
+ * upstream's fp32 torch arithmetic on the GPU.  m_prev is read only for order 2.
+ * Aliasing: x_prev may alias x; no other pointers may overlap (m_store and m_prev are two slots of the caller's ring). */
+int mkd_dpm_update(const float* x, const float* eps, int cfg, float cfg_scale, float alpha_s, float sigma_s, float* m_store,
+                   int order, const float* m_prev, float sigma_ratio, float phi, float half_phi, float inv_r0, float* x_prev,
+                   int64_t n, mkd_stream_t stream);
+
+/* The same update with x_prev written to n_peers (1..8) destinations, as mkd_ddim_update_peers: the last step of a
+ * batch-sharded DPM-Solver run stores its slice of the all-gathered result into every rank's gather buffer.  Values are
+ * bit-identical to mkd_dpm_update. */
+int mkd_dpm_update_peers(const float* x, const float* eps, int cfg, float cfg_scale, float alpha_s, float sigma_s,
+                         float* m_store, int order, const float* m_prev, float sigma_ratio, float phi, float half_phi,
+                         float inv_r0, float* const* x_prev_peers, int n_peers, int64_t n, mkd_stream_t stream);
+
 /* ---- layout / small elementwise ---------------------------------------------------------------------------
  * NCHW fp32 (the reference boundary layout, makeup_diffuse.py:152) <-> NHWC working layout. */
 int mkd_nchw_to_nhwc(const float* src, void* dst, int dtype, int N, int C, int H, int W, int ld_dst,
@@ -109,6 +135,11 @@ int mkd_nhwc_to_nchw(const void* src, float* dst, int dtype, int N, int C, int H
 /* upstream timestep_embedding(): out[b, :] = [cos(t_b f_k), sin(t_b f_k)], optionally followed by nothing. */
 int mkd_timestep_embedding(const int64_t* t, void* out, int dtype, int B, int dim, float max_period,
                            mkd_stream_t stream);
+/* The same embedding of fp32 timesteps (ABI v12): upstream's `t[:, None].float() * freqs` takes fractional t as they
+ * are (DPM-Solver feeds the model (t_continuous - 1/N) * 1000).  For integer t below 2^24 the result is bit-identical to
+ * mkd_timestep_embedding's. */
+int mkd_timestep_embedding_f32(const float* t, void* out, int dtype, int B, int dim, float max_period,
+                               mkd_stream_t stream);
 /* y = silu(x) on n contiguous elements (ResBlock emb_layers.0, time_embed.1). */
 int mkd_silu(const void* x, void* y, int dtype, int64_t n, mkd_stream_t stream);
 /* GEGLU (upstream ldm.modules.attention.GEGLU): y[m, j] = x[m, j] * gelu_erf(x[m, inner + j]). */

@@ -14,7 +14,7 @@ LIB_PATH = os.path.join(_HERE, "libmkd_b200.so")
 MKD_BF16, MKD_F32 = 0, 1
 ACT_NONE, ACT_SILU, ACT_GEGLU = 0, 1, 2
 PATH_AUTO, PATH_GENERIC, PATH_TCGEN05, PATH_TCGEN05_SINGLE, PATH_TCGEN05_PAIR = 0, 1, 2, 3, 4
-ABI_VERSION = 11
+ABI_VERSION = 12
 
 
 class ConvDesc(C.Structure):
@@ -54,9 +54,12 @@ PROTOTYPES = {
     "mkd_ddim_update_peers": (_i, [_vp, _vp, _i, _f, _vp, _f, _f, _f, _f, _f, _f, _vp, _i, _vp, _i64, _vp]),
     "mkd_plms_update": (_i, [_vp, _vp, _i, _f, _vp, _i, _vp, _vp, _vp, _f, _f, _f, _f, _vp, _vp, _i64, _vp]),
     "mkd_plms_update_peers": (_i, [_vp, _vp, _i, _f, _vp, _i, _vp, _vp, _vp, _f, _f, _f, _f, _vp, _i, _vp, _i64, _vp]),
+    "mkd_dpm_update": (_i, [_vp, _vp, _i, _f, _f, _f, _vp, _i, _vp, _f, _f, _f, _f, _vp, _i64, _vp]),
+    "mkd_dpm_update_peers": (_i, [_vp, _vp, _i, _f, _f, _f, _vp, _i, _vp, _f, _f, _f, _f, _vp, _i, _i64, _vp]),
     "mkd_nchw_to_nhwc": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _i, _vp]),
     "mkd_nhwc_to_nchw": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _i, _vp]),
     "mkd_timestep_embedding": (_i, [_vp, _vp, _i, _i, _i, _f, _vp]),
+    "mkd_timestep_embedding_f32": (_i, [_vp, _vp, _i, _i, _i, _f, _vp]),
     "mkd_silu": (_i, [_vp, _vp, _i, _i64, _vp]),
     "mkd_geglu": (_i, [_vp, _vp, _i, _i64, _i, _i, _i, _vp]),
     "mkd_add": (_i, [_vp, _vp, _vp, _i, _i64, _i, _i, _i, _i, _vp]),

@@ -1,4 +1,4 @@
-// Probes, the fused DDIM update (+CFG) kernel, layout conversion and the small elementwise kernels.
+// Probes, the fused DDIM / PLMS / DPM-Solver update (+CFG) kernels, layout conversion and the small elementwise kernels.
 #include <math.h>
 #include <stdarg.h>
 #include <stdlib.h>
@@ -226,6 +226,81 @@ extern "C" int mkd_plms_update_peers(const float* x, const float* eps, int cfg, 
 }
 
 // ---------------------------------------------------------------------------------------------------------
+// DPM-Solver++ multistep update (upstream dpm_solver.py, predict_x0=True, solver_type 'dpm_solver'): the CFG combine,
+// the data prediction m_k at the evaluated time, its store into the sampler's two-slot ring and the order-1 or order-2
+// step to the next time, in one pass.  x / x_prev carry no __restrict__ (the header allows x_prev == x); each thread reads
+// every input element before it stores its own.  The data prediction is a true division by alpha_s, as upstream's
+// tensor / tensor; every other scalar arrives precomputed from upstream's torch expressions.
+// ---------------------------------------------------------------------------------------------------------
+template <int NP>
+__global__ void dpm_update_kernel(const float* x, const float* __restrict__ eps, int cfg, float cfg_scale, float alpha_s,
+                                  float sigma_s, float* __restrict__ m_store, int order, const float* __restrict__ m_prev,
+                                  float ratio, float phi, float half_phi, float inv_r0, PeerPtrs out, int64_t n) {
+  pdl_wait();
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+    float e = eps[i];
+    if (cfg) e = __fadd_rn(e, __fmul_rn(cfg_scale, __fsub_rn(eps[n + i], e)));  // noise_uncond + s * (noise - noise_uncond)
+    float xv = x[i];
+    float m = __fdiv_rn(__fsub_rn(xv, __fmul_rn(sigma_s, e)), alpha_s);  // data_prediction_fn
+    float xp = __fsub_rn(__fmul_rn(ratio, xv), __fmul_rn(phi, m));       // (sigma_t / sigma_s) x - (alpha_t phi) m_k
+    if (order == 2) {
+      float d = __fmul_rn(inv_r0, __fsub_rn(m, m_prev[i]));            // D1_0 = (1 / r0) (m_k - m_{k-1})
+      xp = __fsub_rn(xp, __fmul_rn(half_phi, d));                      //   - (0.5 alpha_t phi) D1_0
+    }
+    if (m_store) m_store[i] = m;
+#pragma unroll
+    for (int r = 0; r < NP; ++r) out.p[r][i] = xp;
+  }
+}
+
+static int dpm_launch(const float* x, const float* eps, int cfg, float cfg_scale, float alpha_s, float sigma_s,
+                      float* m_store, int order, const float* m_prev, float ratio, float phi, float half_phi, float inv_r0,
+                      const PeerPtrs& pp, int n_peers, int64_t n, mkd_stream_t stream, const char* who) {
+  MKD_REQUIRE(x && eps && n >= 0, MKD_E_INVALID, "%s: null pointer or negative n", who);
+  MKD_REQUIRE(order == 1 || order == 2, MKD_E_INVALID, "%s: order=%d must be 1 or 2", who, order);
+  MKD_REQUIRE(order == 1 || m_prev, MKD_E_INVALID, "%s: order 2 needs m_prev", who);
+  for (int r = 0; r < n_peers; ++r) MKD_REQUIRE(pp.p[r] != nullptr, MKD_E_INVALID, "%s: null x_prev pointer %d", who, r);
+  if (n == 0) return MKD_OK;
+  int threads = 256;
+  int blocks = (int)((n + threads - 1) / threads);
+  if (blocks > 148 * 8) blocks = 148 * 8;
+  cudaStream_t st = (cudaStream_t)stream;
+#define MKD_DPM_CASE(NP)                                                                                                \
+  case NP:                                                                                                              \
+    MKD_LAUNCH_OK(launch_pdl(dpm_update_kernel<NP>, dim3(blocks), dim3(threads), 0, st, x, eps, cfg, cfg_scale, alpha_s, \
+                             sigma_s, m_store, order, m_prev, ratio, phi, half_phi, inv_r0, pp, n));                    \
+    break;
+  switch (n_peers) {
+    MKD_DPM_CASE(1) MKD_DPM_CASE(2) MKD_DPM_CASE(3) MKD_DPM_CASE(4)
+    MKD_DPM_CASE(5) MKD_DPM_CASE(6) MKD_DPM_CASE(7) MKD_DPM_CASE(8)
+  }
+#undef MKD_DPM_CASE
+  MKD_CHECK_LAUNCH();
+  return MKD_OK;
+}
+
+extern "C" int mkd_dpm_update(const float* x, const float* eps, int cfg, float cfg_scale, float alpha_s, float sigma_s,
+                              float* m_store, int order, const float* m_prev, float sigma_ratio, float phi, float half_phi,
+                              float inv_r0, float* x_prev, int64_t n, mkd_stream_t stream) {
+  PeerPtrs pp = {};
+  pp.p[0] = x_prev;
+  return dpm_launch(x, eps, cfg, cfg_scale, alpha_s, sigma_s, m_store, order, m_prev, sigma_ratio, phi, half_phi, inv_r0,
+                    pp, 1, n, stream, "dpm_update");
+}
+
+extern "C" int mkd_dpm_update_peers(const float* x, const float* eps, int cfg, float cfg_scale, float alpha_s,
+                                    float sigma_s, float* m_store, int order, const float* m_prev, float sigma_ratio,
+                                    float phi, float half_phi, float inv_r0, float* const* x_prev_peers, int n_peers,
+                                    int64_t n, mkd_stream_t stream) {
+  MKD_REQUIRE(x_prev_peers, MKD_E_INVALID, "dpm_update_peers: null peer array");
+  MKD_REQUIRE(n_peers >= 1 && n_peers <= 8, MKD_E_INVALID, "dpm_update_peers: n_peers=%d must be 1..8 (one box)", n_peers);
+  PeerPtrs pp = {};
+  for (int r = 0; r < n_peers; ++r) pp.p[r] = x_prev_peers[r];  // host array of device pointers
+  return dpm_launch(x, eps, cfg, cfg_scale, alpha_s, sigma_s, m_store, order, m_prev, sigma_ratio, phi, half_phi, inv_r0,
+                    pp, n_peers, n, stream, "dpm_update_peers");
+}
+
+// ---------------------------------------------------------------------------------------------------------
 // NCHW fp32 <-> NHWC T through a 32x32 smem transpose tile (coalesced on both sides).
 // ---------------------------------------------------------------------------------------------------------
 template <typename T>
@@ -308,6 +383,35 @@ extern "C" int mkd_timestep_embedding(const int64_t* t, void* out, int dtype, in
     MKD_LAUNCH_OK(launch_pdl(timestep_embedding_kernel<bf16>, dim3(blocks), dim3(threads), 0, (cudaStream_t)stream, t, (bf16*)out, B, dim, nl));
   else
     MKD_LAUNCH_OK(launch_pdl(timestep_embedding_kernel<float>, dim3(blocks), dim3(threads), 0, (cudaStream_t)stream, t, (float*)out, B, dim, nl));
+  MKD_CHECK_LAUNCH();
+  return MKD_OK;
+}
+
+// fp32 timesteps (DPM-Solver's fractional model times): upstream's t.float() * freqs with t as given.  The body is the
+// int64 kernel's with (float)t[b] already a float, so integer t below 2^24 give the same bits.
+template <typename T>
+__global__ void timestep_embedding_f32_kernel(const float* __restrict__ t, T* __restrict__ out, int B, int dim,
+                                              float neg_log_mp) {
+  pdl_wait();
+  int half = dim / 2;
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < B * half; i += gridDim.x * blockDim.x) {
+    int b = i / half, k = i % half;
+    float f = expf(neg_log_mp * (float)k / (float)half);
+    float a = t[b] * f;
+    out[(int64_t)b * dim + k] = from_f<T>(cosf(a));
+    out[(int64_t)b * dim + half + k] = from_f<T>(sinf(a));
+    if ((dim & 1) && k == 0) out[(int64_t)b * dim + dim - 1] = from_f<T>(0.f);
+  }
+}
+extern "C" int mkd_timestep_embedding_f32(const float* t, void* out, int dtype, int B, int dim, float max_period,
+                                          mkd_stream_t stream) {
+  MKD_REQUIRE(t && out && B > 0 && dim >= 2, MKD_E_INVALID, "timestep_embedding_f32: bad args");
+  int n = B * (dim / 2), threads = 128, blocks = (n + threads - 1) / threads;
+  float nl = -logf(max_period);
+  if (dtype == MKD_BF16)
+    MKD_LAUNCH_OK(launch_pdl(timestep_embedding_f32_kernel<bf16>, dim3(blocks), dim3(threads), 0, (cudaStream_t)stream, t, (bf16*)out, B, dim, nl));
+  else
+    MKD_LAUNCH_OK(launch_pdl(timestep_embedding_f32_kernel<float>, dim3(blocks), dim3(threads), 0, (cudaStream_t)stream, t, (float*)out, B, dim, nl));
   MKD_CHECK_LAUNCH();
   return MKD_OK;
 }

@@ -13,7 +13,8 @@ only data-path collective is ONE all-gather of the final latents over NVLink 5 /
 
 ``sample_sharded`` runs the DDIM sampling loop this way; ``encode_sharded`` the DDIM inversion (x_0 -> x_t) of a
 dataset's latents, whose last inversion step writes into the gather buffer the same way; ``sample_plms_sharded`` the PLMS
-sampling loop (B200PLMSSampler), whose last update kernel (``mkd_plms_update[_peers]``) does the same.
+sampling loop (B200PLMSSampler), whose last update kernel (``mkd_plms_update[_peers]``) does the same;
+``sample_dpm_sharded`` the DPM-Solver++ loop (B200DPMSolverSampler, ``mkd_dpm_update[_peers]``) likewise.
 """
 from __future__ import annotations
 
@@ -98,18 +99,33 @@ def sample_sharded(sampler, S, batch_global, shape, cond_local, x_T_local, rank=
     return _gather_end(gathered, mine, hdl, world, group)
 
 
-def sample_plms_sharded(sampler, S, batch_global, shape, cond_local, x_T_local, rank=0, world=1, group=None,
-                        fused_gather=False, **kw):
-    """PLMS-sample this rank's chunk (B200PLMSSampler.sample) and all-gather the final latents.
-
-    Arguments as sample_sharded; kw goes to sample (eta, guidance, callbacks).  Returns the [batch_global, C, H, W] latents
-    on every rank.  Requires equal chunk sizes when world > 1."""
+def _sample_with_sharded(sampler, S, batch_global, shape, cond_local, x_T_local, rank, world, group, fused_gather, kw):
+    """run ``sampler.sample`` on this rank's chunk with its last update writing into the gather buffer; the samplers whose
+    ``sample`` takes ``out=`` / ``peer_ptrs=`` (B200PLMSSampler, B200DPMSolverSampler)"""
     lo, hi = shard_bounds(batch_global, rank, world)
     gathered, mine, hdl, peer_ptrs = _gather_begin(batch_global, lo, hi, tuple(shape), x_T_local.device, world, group,
                                                    fused_gather)
     kw.setdefault("verbose", False)
     sampler.sample(S, hi - lo, tuple(shape), cond_local, x_T=x_T_local, out=mine, peer_ptrs=peer_ptrs, **kw)
     return _gather_end(gathered, mine, hdl, world, group)
+
+
+def sample_plms_sharded(sampler, S, batch_global, shape, cond_local, x_T_local, rank=0, world=1, group=None,
+                        fused_gather=False, **kw):
+    """PLMS-sample this rank's chunk (B200PLMSSampler.sample) and all-gather the final latents.
+
+    Arguments as sample_sharded; kw goes to sample (eta, guidance, callbacks).  Returns the [batch_global, C, H, W] latents
+    on every rank.  Requires equal chunk sizes when world > 1."""
+    return _sample_with_sharded(sampler, S, batch_global, shape, cond_local, x_T_local, rank, world, group, fused_gather, kw)
+
+
+def sample_dpm_sharded(sampler, S, batch_global, shape, cond_local, x_T_local, rank=0, world=1, group=None,
+                       fused_gather=False, **kw):
+    """DPM-Solver-sample this rank's chunk (B200DPMSolverSampler.sample) and all-gather the final latents.
+
+    Arguments as sample_sharded; kw goes to sample (guidance).  Returns the [batch_global, C, H, W] latents on every rank.
+    Requires equal chunk sizes when world > 1."""
+    return _sample_with_sharded(sampler, S, batch_global, shape, cond_local, x_T_local, rank, world, group, fused_gather, kw)
 
 
 def encode_sharded(sampler, t_enc, batch_global, x0_local, cond_local, rank=0, world=1, group=None, fused_gather=False,

@@ -17,7 +17,7 @@ import numpy as np
 import torch
 
 from . import ops
-from .nets import B200ControlNet, B200ControlledUnet, B200GroupedTrunk
+from .nets import B200ControlNet, B200ControlledUnet, B200GroupedTrunk, timesteps_for_embedding
 
 
 class _Wrapper:
@@ -98,31 +98,40 @@ class B200ControlLDM:
     # uses ONE t for the whole batch (cddim.py:86-89 / upstream ddim_sampling: ts = torch.full((b,), step)), so the sampler
     # asks for all S of them at once — two MLP chains over S rows instead of S x 2 chains over the batch, each streaming
     # ~85 MB of weights for 16 rows — and selects one row per step.  apply_model(x, t, cond) without a selected step
-    # computes the embeddings from its t argument as before.
+    # computes the embeddings from its t argument as before.  A DPM-Solver loop feeds fractional model times: integer
+    # timesteps key the table as ints (the DDIM / PLMS loops, unchanged), every other value as its exact fp32 value.
+    @staticmethod
+    def _time_key(v):
+        if isinstance(v, (int, np.integer)) or (torch.is_tensor(v) and not v.is_floating_point()):
+            return int(v)
+        return float(np.float32(v))
+
     def precompute_time_embeddings(self, values):
-        vals = tuple(int(v) for v in values)
+        vals = tuple(self._time_key(v) for v in values)
         tb = self._emb_table
         if tb is not None and tb["vals"] == vals and tb["epoch"] == self._weights_epoch:
             return
         un, cn = self.model.diffusion_model, self.control_model
-        tv = torch.tensor(vals, dtype=torch.int64, device=self._device)
+        integer = all(isinstance(v, int) for v in vals)
+        tv = torch.tensor(vals, dtype=torch.int64 if integer else torch.float32, device=self._device)
         tab = torch.zeros(len(vals), 2, un._emb_total, dtype=self.dtype, device=self._device)
         un._time_embedding(tv, len(vals), out=tab[:, 0])
         cn._time_embedding(tv, len(vals), out=tab[:, 1, :cn._emb_total])
         self._emb_table = {"vals": vals, "row": {v: i for i, v in enumerate(vals)}, "tab": tab, "epoch": self._weights_epoch}
 
     def set_step(self, t_value, rows=None):
-        """select the precomputed embeddings of timestep ``t_value`` for the next apply_model calls on ``rows`` batch rows
-        (all at that timestep); ``None`` returns to computing them from the ``t`` argument.  Returns whether a row is selected."""
+        """select the precomputed embeddings of timestep ``t_value`` (an int, or a float selecting the row of its fp32 value)
+        for the next apply_model calls on ``rows`` batch rows (all at that timestep); ``None`` returns to computing them from
+        the ``t`` argument.  Returns whether a row is selected."""
         self._emb_rows = None
         tb = self._emb_table
-        if t_value is None or tb is None or tb["epoch"] != self._weights_epoch or int(t_value) not in tb["row"]:
+        if t_value is None or tb is None or tb["epoch"] != self._weights_epoch or self._time_key(t_value) not in tb["row"]:
             return False
         tot = tb["tab"].shape[2]
         buf = self._emb_bufs.get(rows)
         if buf is None:
             buf = self._emb_bufs[rows] = torch.empty(2 * rows, tot, dtype=self.dtype, device=self._device)
-        buf.view(2, rows, tot).copy_(tb["tab"][tb["row"][int(t_value)]][:, None, :].expand(2, rows, tot))
+        buf.view(2, rows, tot).copy_(tb["tab"][tb["row"][self._time_key(t_value)]][:, None, :].expand(2, rows, tot))
         self._emb_rows = rows
         return True
 
@@ -193,7 +202,7 @@ class B200ControlLDM:
         use_cn = cond["c_concat"] is not None
         grouped = use_cn and self._use_grouped(N, H, W)
         prep = self._prepare(cond, grouped)
-        t = t.to(torch.int64).contiguous()
+        t = timesteps_for_embedding(t)
         emb2 = self._emb_bufs[N] if self._emb_rows == N else None  # [UNet rows | ControlNet rows] of the selected step
         emb_un = None if emb2 is None else emb2[:N]
         emb_cn = None if emb2 is None else emb2[N:, :cn._emb_total]

@@ -30,6 +30,13 @@ from . import ops
 _SPLITK_WS_BYTES = 96 << 20
 
 
+def timesteps_for_embedding(t):
+    """the timestep tensor the embedding kernels take: integer timesteps as int64 (mkd_timestep_embedding), floating ones
+    as fp32 (mkd_timestep_embedding_f32), so a fractional t is not truncated.  For integers below 2^24 both give the
+    same bits."""
+    return (t.to(torch.float32) if t.is_floating_point() else t.to(torch.int64)).contiguous()
+
+
 class Act:
     """A trunk tensor of the bf16 path, stored up to twice:
     ``lo`` — activation dtype (bf16), what tensor-core A operands and the decoder's concat slots read;
@@ -315,9 +322,13 @@ class _Net(nn.Module):
 
     def _time_embedding(self, t, B, out=None):
         """emb = time_embed(timestep_embedding(t)); returns silu(emb) @ W_all + b_all for every ResBlock at once
-        (into ``out``, a [B, _emb_total] view, when given)."""
+        (into ``out``, a [B, _emb_total] view, when given).  t: int64 timesteps, or fp32 ones (fractional values as they
+        are, as upstream's t.float() takes them) — see timesteps_for_embedding."""
         te = self._buf("t_emb", B, self.mc)
-        ops.timestep_embedding(t, te)
+        if t.is_floating_point():
+            ops.timestep_embedding_f32(t, te)
+        else:
+            ops.timestep_embedding(t, te)
         e1 = self._buf("te1", B, self.ted)
         self._linear(te, "te0", e1, act=L.ACT_SILU)
         e2 = self._buf("te2", B, self.ted)
@@ -669,8 +680,7 @@ class B200ControlNet(_Net):
         assert self._loaded, "load_state_dict() first"
         N, _, H, W = x.shape
         xin = self._x_in(x)
-        outs = self.run(xin, self.hint_features(hint), timesteps.to(torch.int64).contiguous(),
-                        self.context_kv(context), N, H, W)
+        outs = self.run(xin, self.hint_features(hint), timesteps_for_embedding(timesteps), self.context_kv(context), N, H, W)
         res = []
         for o, h, w in outs:
             t = torch.empty(N, o.shape[1], h, w, dtype=torch.float32, device=o.device)
@@ -824,7 +834,7 @@ class B200ControlledUnet(_Net):
         N, _, H, W = x.shape
         ctx_kv = self.context_kv(context)
         xin = self._x_in(x)
-        slots = self.encode(xin, timesteps.to(torch.int64).contiguous(), ctx_kv, N, H, W)
+        slots = self.encode(xin, timesteps_for_embedding(timesteps), ctx_kv, N, H, W)
         if control is not None:
             idx = [len(slots) - 1] if only_mid_control else range(len(slots))
             for j in idx:

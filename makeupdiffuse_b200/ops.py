@@ -120,6 +120,33 @@ def plms_update(x, eps, x_prev, *, mode, history=(), e_store=None, sqrt_one_minu
     L.check(L.load().mkd_plms_update(*head, x_prev.data_ptr(), _p(pred_x0), n, _stream()), "plms_update")
 
 
+def dpm_update(x, eps, x_prev, *, alpha_s, sigma_s, sigma_ratio, phi, order=1, m_prev=None, half_phi=0.0, inv_r0=0.0,
+               m_store=None, cfg_scale=None, peer_ptrs=None):
+    """One DPM-Solver++ multistep update (upstream dpm_solver.py, predict_x0=True, after one model call): eps holds n values,
+    or 2n ([uncond; cond]) when cfg_scale is given; the data prediction m = (x - sigma_s * e) / alpha_s goes to m_store
+    when given; order 1 steps with m alone, order 2 also with the previous data prediction m_prev.  The scalars come from
+    upstream's expressions (mkd_dpm_update in include/mkd_b200.h)."""
+    n = x.numel()
+    if order not in (1, 2) or (order == 2) != (m_prev is not None):
+        raise ValueError("dpm_update: order 1 takes no m_prev, order 2 needs it")
+    for t in (x, eps, x_prev, m_store, m_prev):
+        if t is not None and (t.dtype != torch.float32 or not t.is_contiguous() or not t.is_cuda):
+            raise ValueError("dpm_update works on contiguous fp32 CUDA latents")
+    for t in (x_prev, m_store, m_prev):
+        if t is not None and t.numel() != n:
+            raise ValueError("dpm_update: every latent-sized tensor must hold x.numel() values")
+    cfg = cfg_scale is not None
+    if eps.numel() != (2 * n if cfg else n):
+        raise ValueError("eps has the wrong number of elements")
+    head = (x.data_ptr(), eps.data_ptr(), int(cfg), float(cfg_scale or 0.0), float(alpha_s), float(sigma_s), _p(m_store),
+            int(order), _p(m_prev), float(sigma_ratio), float(phi), float(half_phi), float(inv_r0))
+    if peer_ptrs is not None:  # x_prev goes to every rank's gather buffer (mkd_dpm_update_peers); x_prev = own slice
+        arr = (C.c_void_p * len(peer_ptrs))(*[int(p) for p in peer_ptrs])
+        L.check(L.load().mkd_dpm_update_peers(*head, arr, len(peer_ptrs), n, _stream()), "dpm_update_peers")
+        return
+    L.check(L.load().mkd_dpm_update(*head, x_prev.data_ptr(), n, _stream()), "dpm_update")
+
+
 @_timed("nchw_to_nhwc", lambda s, d: _nb(s, d))
 def nchw_to_nhwc(src, dst2d):
     N, Cc, H, W = src.shape
@@ -146,6 +173,15 @@ def timestep_embedding(t, out, max_period=10000.0):
     B, dim = out.shape
     L.check(L.load().mkd_timestep_embedding(t.data_ptr(), out.data_ptr(), _dt(out), B, dim, float(max_period), _stream()),
             "timestep_embedding")
+
+
+@_timed("timestep_embedding_f32", None)
+def timestep_embedding_f32(t, out, max_period=10000.0):
+    """upstream timestep_embedding of fp32 timesteps, fractional ones as they are"""
+    assert t.dtype == torch.float32 and t.is_contiguous() and out.is_contiguous()
+    B, dim = out.shape
+    L.check(L.load().mkd_timestep_embedding_f32(t.data_ptr(), out.data_ptr(), _dt(out), B, dim, float(max_period),
+                                                _stream()), "timestep_embedding_f32")
 
 
 @_timed("silu", lambda x, y: _nb(x, y))

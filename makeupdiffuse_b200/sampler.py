@@ -10,7 +10,8 @@ The RNG stream is consumed exactly like the reference: one ``randn(x.shape)`` pe
 (cddim.py:75).  Unlike upstream nothing is force-moved to "cuda": buffers follow ``model.device``.
 
 ``B200PLMSSampler`` (below) is the drop-in for upstream ``PLMSSampler`` on the same machinery, with its own fused update
-kernel (mkd_plms_update).
+kernel (mkd_plms_update); ``B200DPMSolverSampler`` the drop-in for upstream ``DPMSolverSampler`` (DPM-Solver++(2M) at
+fractional model times, one fused mkd_dpm_update per evaluation).
 """
 from __future__ import annotations
 
@@ -139,14 +140,15 @@ class B200DDIMSampler:
         refilled the same tensors in a way torch's version counter does not see.  Loops driven from outside
         (makeupdiffuse_b200.dist.sample_sharded, a caller's own loop over denoising_step) call this themselves.
         steps: the loop's timesteps, when known: the model computes the timestep embeddings of all of them at once, and
-        denoising_step(..., t_value=step) selects one per step."""
+        denoising_step(..., t_value=step) selects one per step.  Integer steps select as ints; fractional model times (the
+        DPM-Solver loop) select by their fp32 value."""
         self._cfg_cache = None
         inv = getattr(self.model, "invalidate_cond_cache", None)
         if inv is not None:
             inv()
         pre = getattr(self.model, "precompute_time_embeddings", None)
         if pre is not None and steps is not None and len(steps):
-            pre([int(v) for v in steps])
+            pre(list(steps))
 
     def p_sample_ddim(self, *a, **k):
         with torch.no_grad():
@@ -174,7 +176,7 @@ class B200DDIMSampler:
     def _eps(self, x, t, c, t_value=None):
         """model.apply_model(x, t, c); with use_cuda_graph the ~10^3 kernel launches of one UNet+ControlNet step are
         captured once per (cond, batch shape) and replayed (launch-bound otherwise: SURVEY.md §7 hard part 6).
-        t_value: the loop's timestep as a host int when every row of ``t`` holds it (the sampler's own loops): the model
+        t_value: the loop's timestep as a host int (or float) when every row of ``t`` holds it (the sampler's own loops): the model
         then takes the ResBlock timestep embeddings from the table computed at the start of the loop (begin_loop(steps))
         instead of running the two embedding MLPs again."""
         set_step = getattr(self.model, "set_step", None)
@@ -200,6 +202,7 @@ class B200DDIMSampler:
                # a graph holds raw pointers and the launch structure of the moment it was captured: reloaded weights
                # (new tensors), another stream layout or another GroupNorm path need a new capture
                getattr(m, "_weights_epoch", 0), getattr(m, "concurrent", None), getattr(m, "grouped", None), emb_selected,
+               t.dtype,  # the captured copy_ into the graph's t would cast a fractional fp32 t to int64
                tuple((getattr(n, "fused_gn_stats", None), getattr(n, "fuse_gn_tail", None)) for n in nets))
         if g is None or g["key"] != key:
             sx, st = x.clone(), t.clone()
@@ -479,3 +482,141 @@ class B200PLMSSampler(B200DDIMSampler):
                         peer_ptrs=peer_ptrs, **coef)
         draw()
         return x_prev, pred_x0, e_t
+
+
+def _cond_batch(c):
+    """rows of the first conditioning tensor (upstream's batch-size check reads conditioning[first key].shape[0]; here
+    a list value, as in this model's dict-of-lists cond, gives its first tensor)"""
+    v = c[next(iter(c))] if isinstance(c, dict) else c
+    if isinstance(v, list):
+        v = v[0] if v else None
+    return None if v is None else v.shape[0]
+
+
+def _elementwise(fn, v):
+    """fn(v) for an elementwise torch function of a 1-D tensor.  On the CPU it is applied one element at a time: torch's
+    vectorised CPU exp / log / expm1 can differ by an ulp from the scalar ones, which are the ones upstream's per-step
+    [batch]-sized tensors take (below 16 rows).  On CUDA an element's value does not depend on its position."""
+    if v.is_cuda:
+        return fn(v)
+    return torch.cat([fn(v[k:k + 1]) for k in range(v.shape[0])])
+
+
+class B200DPMSolverSampler(B200DDIMSampler):
+    """Drop-in for upstream ``ldm.models.diffusion.dpm_solver.DPMSolverSampler``: DPM-Solver++(2M) — upstream's fixed
+    configuration: ``NoiseScheduleVP('discrete', alphas_cumprod)``, noise model with classifier-free guidance,
+    ``predict_x0=True``, ``skip_type='time_uniform'``, ``method='multistep'``, ``order=2``, ``lower_order_final=True``.
+    A run of S steps makes S model evaluations at the fractional model times (t - 1/N) * 1000 and draws no noise when
+    ``x_T`` is given.  Per evaluation: one graph-replayed UNet+ControlNet call, then one fused kernel (mkd_dpm_update)
+    for the CFG combine, the data prediction (kept in a ring of two device buffers) and the order-1 / order-2 step to the
+    next time.  One deliberate superset: the guided call and the batch-size check accept this model's dict-of-lists
+    cond (upstream's ``torch.cat([uc, c])`` and ``conditioning[key].shape`` take bare tensors only)."""
+
+    order = 2
+
+    # ---- upstream NoiseScheduleVP('discrete', alphas_cumprod=...) ------------------------------------------------------
+    def _noise_schedule(self):
+        """(t_array [1, N], log_alpha_array [1, N]) on the model's device: log_alpha = 0.5 * log(alphas_cumprod) on the
+        fp32 device schedule, t_array = linspace(0, 1, N + 1)[1:] built on the CPU"""
+        ac = self.model.alphas_cumprod.detach().to(torch.float32).to(self.model.device)
+        N = ac.shape[0]
+        t_array = torch.linspace(0., 1., N + 1)[1:].reshape((1, -1)).to(ac.device)
+        return t_array, (0.5 * torch.log(ac)).reshape((1, -1))
+
+    @staticmethod
+    def _interpolate(x, xp, yp):
+        """upstream interpolate_fn: the piecewise-linear function through (xp, yp), extended linearly beyond the ends;
+        x [N, 1], xp / yp [1, K]"""
+        N, K = x.shape[0], xp.shape[1]
+        all_x = torch.cat([x.unsqueeze(2), xp.unsqueeze(0).repeat((N, 1, 1))], dim=2)
+        sorted_all_x, x_indices = torch.sort(all_x, dim=2)
+        x_idx = torch.argmin(x_indices, dim=2)
+        cand_start_idx = x_idx - 1
+        start_idx = torch.where(torch.eq(x_idx, 0), torch.tensor(1, device=x.device),
+                                torch.where(torch.eq(x_idx, K), torch.tensor(K - 2, device=x.device), cand_start_idx))
+        end_idx = torch.where(torch.eq(start_idx, cand_start_idx), start_idx + 2, start_idx + 1)
+        start_x = torch.gather(sorted_all_x, dim=2, index=start_idx.unsqueeze(2)).squeeze(2)
+        end_x = torch.gather(sorted_all_x, dim=2, index=end_idx.unsqueeze(2)).squeeze(2)
+        start_idx2 = torch.where(torch.eq(x_idx, 0), torch.tensor(0, device=x.device),
+                                 torch.where(torch.eq(x_idx, K), torch.tensor(K - 2, device=x.device), cand_start_idx))
+        y_positions_expanded = yp.unsqueeze(0).expand(N, -1, -1)
+        start_y = torch.gather(y_positions_expanded, dim=2, index=start_idx2.unsqueeze(2)).squeeze(2)
+        end_y = torch.gather(y_positions_expanded, dim=2, index=(start_idx2 + 1).unsqueeze(2)).squeeze(2)
+        return start_y + (x - start_x) * (end_y - start_y) / (end_x - start_x)
+
+    def _loop_scalars(self, S):
+        """Everything a run of S steps needs, once per loop and on the model's device, with upstream's expressions:
+        the model times and, per evaluation k (at t_k, stepping to t_{k+1}), the arguments of mkd_dpm_update."""
+        dev = self.model.device
+        t_array, log_alpha_array = self._noise_schedule()
+        N = t_array.shape[1]
+        # DPMSolver.sample / get_time_steps('time_uniform'): linspace(t_T, t_0, S + 1) on the CPU, then to the device
+        times = torch.linspace(1., 1. / N, S + 1).to(dev)
+        model_times = (times[:S] - 1. / N) * 1000.  # model_wrapper.get_model_input_time
+
+        def marginals(t):  # marginal_log_mean_coeff -> marginal_alpha, marginal_std, marginal_lambda
+            lmc = self._interpolate(t.reshape((-1, 1)), t_array, log_alpha_array).reshape((-1))
+            alpha = torch.exp(lmc)
+            sigma = torch.sqrt(1. - torch.exp(2. * lmc))
+            lam = lmc - 0.5 * torch.log(1. - torch.exp(2. * lmc))
+            return torch.stack([alpha, sigma, lam])
+
+        alpha, sigma, lam = _elementwise(lambda t: marginals(t).t(), times).t()
+        h = lam[1:] - lam[:-1]                               # h of the step t_k -> t_{k+1}
+        ratio = sigma[1:] / sigma[:-1]                       # sigma_t / sigma_s
+        phi1 = alpha[1:] * _elementwise(torch.expm1, -h)     # dpm_solver_first_update: alpha_t * expm1(-h)
+        phi2 = alpha[1:] * (_elementwise(torch.exp, -h) - 1.)  # multistep_dpm_solver_second_update
+        half2 = 0.5 * phi2
+        r0 = torch.cat([h[:1], h[:-1] / h[1:]])              # h_0 / h, with h_0 = lambda_prev_0 - lambda_prev_1 (k >= 1)
+        inv_r0 = 1. / r0
+        cols = torch.stack([alpha[:S], sigma[:S], ratio, phi1, phi2, half2, inv_r0], 1).tolist()
+        steps = []
+        for k, (a_s, s_s, rt, p1, p2, hp2, ir0) in enumerate(cols):
+            # the first step is order 1; with lower_order_final the last one too when S < 15
+            order = 1 if k == 0 or (S < 15 and k == S - 1) else self.order
+            steps.append(dict(alpha_s=a_s, sigma_s=s_s, sigma_ratio=rt, order=order, phi=p1 if order == 1 else p2,
+                              half_phi=0.0 if order == 1 else hp2, inv_r0=0.0 if order == 1 else ir0))
+        return model_times.tolist(), steps
+
+    @torch.no_grad()
+    def sample(self, S, batch_size, shape, conditioning=None, callback=None, normals_sequence=None, img_callback=None,
+               quantize_x0=False, eta=0.0, mask=None, x0=None, temperature=1.0, noise_dropout=0.0, score_corrector=None,
+               corrector_kwargs=None, verbose=True, x_T=None, log_every_t=100, unconditional_guidance_scale=1.0,
+               unconditional_conditioning=None, out=None, peer_ptrs=None, **kwargs):
+        """upstream DPMSolverSampler.sample: returns (x, None).  Arguments upstream ignores (eta, mask, callbacks, ...)
+        are ignored.  ``out`` / ``peer_ptrs`` (extensions, optional): as in denoising_step, for the LAST update only."""
+        m = self.model
+        if m.parameterization != "eps":
+            raise NotImplementedError("B200 path implements the yaml's parameterization: eps (yaml:50)")
+        if conditioning is not None:
+            cbs = _cond_batch(conditioning)
+            if cbs is not None and cbs != batch_size:
+                print(f"Warning: Got {cbs} conditionings but batch-size is {batch_size}")
+        C, H, W = shape
+        size = (batch_size, C, H, W)
+        if verbose:
+            print(f"Data shape for DPM-Solver sampling is {size}, sampling steps {S}")
+        dev = m.device
+        img = torch.randn(size, device=dev) if x_T is None else x_T
+        assert S >= self.order  # upstream DPMSolver.sample: assert steps >= order
+        model_times, steps = self._loop_scalars(S)
+        self.begin_loop(model_times)
+        cfg = not (unconditional_conditioning is None or unconditional_guidance_scale == 1.0)
+        cc = self._cfg_cond(conditioning, unconditional_conditioning) if cfg else conditioning
+        scale = float(unconditional_guidance_scale) if cfg else None
+        x = img.float().contiguous()
+        ring = torch.empty((2, *x.shape), device=x.device, dtype=torch.float32)  # data predictions m_k, slot k % 2
+        b = x.shape[0]
+        for k, (tv, st) in enumerate(zip(model_times, steps)):
+            t = torch.full((b,), tv, device=x.device, dtype=torch.float32)
+            if not cfg:
+                e = self._eps(x, t, conditioning, t_value=tv)
+            else:
+                e = self._eps(torch.cat([x] * 2), torch.cat([t] * 2), cc, t_value=tv)
+            last = k == S - 1
+            x_next = out if (last and out is not None) else torch.empty_like(x)
+            ops.dpm_update(x, e.contiguous(), x_next, m_store=ring[k % 2],
+                           m_prev=ring[(k - 1) % 2] if st["order"] == 2 else None, cfg_scale=scale,
+                           peer_ptrs=peer_ptrs if last else None, **st)
+            x = x_next
+        return x.to(dev), None
