@@ -31,7 +31,7 @@
 extern "C" {
 #endif
 
-#define MKD_ABI_VERSION 12
+#define MKD_ABI_VERSION 13
 
 typedef void* mkd_stream_t; /* cudaStream_t */
 
@@ -125,6 +125,32 @@ int mkd_dpm_update(const float* x, const float* eps, int cfg, float cfg_scale, f
 int mkd_dpm_update_peers(const float* x, const float* eps, int cfg, float cfg_scale, float alpha_s, float sigma_s,
                          float* m_store, int order, const float* m_prev, float sigma_ratio, float phi, float half_phi,
                          float inv_r0, float* const* x_prev_peers, int n_peers, int64_t n, mkd_stream_t stream);
+
+/* ---- DDPM ancestral step (ABI v13) ------------------------------------------------------------------------------
+ * replaces upstream ldm/models/diffusion/ddpm.py LatentDiffusion.p_sample after its one model call (p_mean_variance with
+ * eps parameterization, q_posterior, the noise term).  x, eps, noise, x0_out, x_prev: n fp32 values as B rows of n / B;
+ * t: the B rows' timesteps (device int64); the five tables: fp32 device vectors of T entries, indexed by t[row]:
+ *   x_recon = sqrt_recip_ac[t] * x - sqrt_recipm1_ac[t] * eps                         (predict_start_from_noise)
+ *   x_recon = clamp(x_recon, -1, 1)                                                   (when clip; NaN stays NaN)
+ *   x0_out  = x_recon                                                                 (skipped when x0_out is NULL)
+ *   mean    = coef1[t] * x_recon + coef2[t] * x                 (posterior_mean_coef1 / posterior_mean_coef2)
+ *   x_prev  = mean + s * (noise * temperature)   (s = sigma[t], or 0 where t == 0: nonzero_mask)
+ * sigma is the caller's exp(0.5 * posterior_log_variance_clipped), evaluated with torch on the device.  Every product
+ * and sum is rounded separately in upstream's order (no FMA contraction), so the result is bit-identical to upstream's
+ * fp32 torch arithmetic on the GPU.  A t outside [0, T) gives NaN in its row.
+ * Aliasing: x_prev may alias x; no other pointers may overlap. */
+int mkd_ddpm_update(const float* x, const float* eps, const int64_t* t, int B, const float* sqrt_recip_ac,
+                    const float* sqrt_recipm1_ac, const float* coef1, const float* coef2, const float* sigma, int T,
+                    int clip, const float* noise, float temperature, float* x0_out, float* x_prev, int64_t n,
+                    mkd_stream_t stream);
+
+/* The same step with x_prev written to n_peers (1..8) destinations, as mkd_ddim_update_peers: the last step of a
+ * batch-sharded DDPM run stores its slice of the all-gathered result into every rank's gather buffer.  Values are
+ * bit-identical to mkd_ddpm_update. */
+int mkd_ddpm_update_peers(const float* x, const float* eps, const int64_t* t, int B, const float* sqrt_recip_ac,
+                          const float* sqrt_recipm1_ac, const float* coef1, const float* coef2, const float* sigma, int T,
+                          int clip, const float* noise, float temperature, float* x0_out, float* const* x_prev_peers,
+                          int n_peers, int64_t n, mkd_stream_t stream);
 
 /* ---- layout / small elementwise ---------------------------------------------------------------------------
  * NCHW fp32 (the reference boundary layout, makeup_diffuse.py:152) <-> NHWC working layout. */

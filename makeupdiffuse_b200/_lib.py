@@ -14,7 +14,7 @@ LIB_PATH = os.path.join(_HERE, "libmkd_b200.so")
 MKD_BF16, MKD_F32 = 0, 1
 ACT_NONE, ACT_SILU, ACT_GEGLU = 0, 1, 2
 PATH_AUTO, PATH_GENERIC, PATH_TCGEN05, PATH_TCGEN05_SINGLE, PATH_TCGEN05_PAIR = 0, 1, 2, 3, 4
-ABI_VERSION = 12
+ABI_VERSION = 13
 
 
 class ConvDesc(C.Structure):
@@ -56,6 +56,8 @@ PROTOTYPES = {
     "mkd_plms_update_peers": (_i, [_vp, _vp, _i, _f, _vp, _i, _vp, _vp, _vp, _f, _f, _f, _f, _vp, _i, _vp, _i64, _vp]),
     "mkd_dpm_update": (_i, [_vp, _vp, _i, _f, _f, _f, _vp, _i, _vp, _f, _f, _f, _f, _vp, _i64, _vp]),
     "mkd_dpm_update_peers": (_i, [_vp, _vp, _i, _f, _f, _f, _vp, _i, _vp, _f, _f, _f, _f, _vp, _i, _i64, _vp]),
+    "mkd_ddpm_update": (_i, [_vp, _vp, _vp, _i, _vp, _vp, _vp, _vp, _vp, _i, _i, _vp, _f, _vp, _vp, _i64, _vp]),
+    "mkd_ddpm_update_peers": (_i, [_vp, _vp, _vp, _i, _vp, _vp, _vp, _vp, _vp, _i, _i, _vp, _f, _vp, _vp, _i, _i64, _vp]),
     "mkd_nchw_to_nhwc": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _i, _vp]),
     "mkd_nhwc_to_nchw": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _i, _vp]),
     "mkd_timestep_embedding": (_i, [_vp, _vp, _i, _i, _i, _f, _vp]),

@@ -1,4 +1,4 @@
-// Probes, the fused DDIM / PLMS / DPM-Solver update (+CFG) kernels, layout conversion and the small elementwise kernels.
+// Probes, the fused DDIM / PLMS / DPM-Solver update (+CFG) kernels, the fused DDPM step, layout conversion and the small elementwise kernels.
 #include <math.h>
 #include <stdarg.h>
 #include <stdlib.h>
@@ -298,6 +298,96 @@ extern "C" int mkd_dpm_update_peers(const float* x, const float* eps, int cfg, f
   for (int r = 0; r < n_peers; ++r) pp.p[r] = x_prev_peers[r];  // host array of device pointers
   return dpm_launch(x, eps, cfg, cfg_scale, alpha_s, sigma_s, m_store, order, m_prev, sigma_ratio, phi, half_phi, inv_r0,
                     pp, n_peers, n, stream, "dpm_update_peers");
+}
+
+// ---------------------------------------------------------------------------------------------------------
+// DDPM ancestral step (upstream ddpm.py p_sample after its model call): predict_start_from_noise, the optional clamp,
+// q_posterior's mean and the noise term, in one pass.  Every row reads its own timestep from the device vector t and
+// its five coefficients from fp32 device tables indexed by it, so the launch is graph-capturable and rows may carry
+// different t.  x / x_prev carry no __restrict__ (the header allows x_prev == x); each thread reads every input element
+// before it stores its own.  A t outside [0, T) yields NaN for that row rather than an out-of-bounds read.
+// ---------------------------------------------------------------------------------------------------------
+struct DdpmTables {
+  const float* sqrt_recip_ac;
+  const float* sqrt_recipm1_ac;
+  const float* coef1;
+  const float* coef2;
+  const float* sigma;
+};
+
+template <int NP>
+__global__ void ddpm_update_kernel(const float* x, const float* __restrict__ eps, const int64_t* __restrict__ t,
+                                   int64_t per_row, DdpmTables tb, int T, int clip, const float* __restrict__ noise,
+                                   float temp, float* __restrict__ x0_out, PeerPtrs out, int64_t n) {
+  pdl_wait();
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t tr = t[i / per_row];
+    const float xv = x[i], e = eps[i], nz = noise[i];
+    float xr = __int_as_float(0x7fffffff), xp = xr;
+    if (tr >= 0 && tr < T) {
+      xr = __fsub_rn(__fmul_rn(tb.sqrt_recip_ac[tr], xv), __fmul_rn(tb.sqrt_recipm1_ac[tr], e));  // x_recon
+      if (clip) xr = xr < -1.f ? -1.f : (xr > 1.f ? 1.f : xr);                                    // clamp_(-1, 1), NaN kept
+      const float mean = __fadd_rn(__fmul_rn(tb.coef1[tr], xr), __fmul_rn(tb.coef2[tr], xv));     // q_posterior mean
+      const float s = tr == 0 ? 0.f : tb.sigma[tr];  // nonzero_mask * exp(0.5 * log_variance): the mask is exact
+      xp = __fadd_rn(mean, __fmul_rn(s, __fmul_rn(nz, temp)));  // mean + (mask * sigma) * (noise * temperature)
+    }
+    if (x0_out) x0_out[i] = xr;
+#pragma unroll
+    for (int r = 0; r < NP; ++r) out.p[r][i] = xp;
+  }
+}
+
+static int ddpm_launch(const float* x, const float* eps, const int64_t* t, int B, const DdpmTables& tb, int T, int clip,
+                       const float* noise, float temperature, float* x0_out, const PeerPtrs& pp, int n_peers, int64_t n,
+                       mkd_stream_t stream, const char* who) {
+  MKD_REQUIRE(x && eps && t && noise && n >= 0, MKD_E_INVALID, "%s: null pointer or negative n", who);
+  MKD_REQUIRE(tb.sqrt_recip_ac && tb.sqrt_recipm1_ac && tb.coef1 && tb.coef2 && tb.sigma && T > 0, MKD_E_INVALID,
+              "%s: null table or T=%d", who, T);
+  MKD_REQUIRE(B >= 1 && n % B == 0, MKD_E_INVALID, "%s: n=%lld is not B=%d rows of equal size", who, (long long)n, B);
+  for (int r = 0; r < n_peers; ++r) MKD_REQUIRE(pp.p[r] != nullptr, MKD_E_INVALID, "%s: null x_prev pointer %d", who, r);
+  if (n == 0) return MKD_OK;
+  int threads = 256;
+  int blocks = (int)((n + threads - 1) / threads);
+  if (blocks > 148 * 8) blocks = 148 * 8;
+  cudaStream_t st = (cudaStream_t)stream;
+  const int64_t per_row = n / B;
+#define MKD_DDPM_CASE(NP)                                                                                              \
+  case NP:                                                                                                             \
+    MKD_LAUNCH_OK(launch_pdl(ddpm_update_kernel<NP>, dim3(blocks), dim3(threads), 0, st, x, eps, t, per_row, tb, T,  \
+                             clip, noise, temperature, x0_out, pp, n));                                               \
+    break;
+  switch (n_peers) {
+    MKD_DDPM_CASE(1) MKD_DDPM_CASE(2) MKD_DDPM_CASE(3) MKD_DDPM_CASE(4)
+    MKD_DDPM_CASE(5) MKD_DDPM_CASE(6) MKD_DDPM_CASE(7) MKD_DDPM_CASE(8)
+  }
+#undef MKD_DDPM_CASE
+  MKD_CHECK_LAUNCH();
+  return MKD_OK;
+}
+
+extern "C" int mkd_ddpm_update(const float* x, const float* eps, const int64_t* t, int B, const float* sqrt_recip_ac,
+                               const float* sqrt_recipm1_ac, const float* coef1, const float* coef2, const float* sigma,
+                               int T, int clip, const float* noise, float temperature, float* x0_out, float* x_prev,
+                               int64_t n, mkd_stream_t stream) {
+  PeerPtrs pp = {};
+  pp.p[0] = x_prev;
+  DdpmTables tb = {sqrt_recip_ac, sqrt_recipm1_ac, coef1, coef2, sigma};
+  return ddpm_launch(x, eps, t, B, tb, T, clip, noise, temperature, x0_out, pp, 1, n, stream, "ddpm_update");
+}
+
+extern "C" int mkd_ddpm_update_peers(const float* x, const float* eps, const int64_t* t, int B,
+                                     const float* sqrt_recip_ac, const float* sqrt_recipm1_ac, const float* coef1,
+                                     const float* coef2, const float* sigma, int T, int clip, const float* noise,
+                                     float temperature, float* x0_out, float* const* x_prev_peers, int n_peers,
+                                     int64_t n, mkd_stream_t stream) {
+  MKD_REQUIRE(x_prev_peers, MKD_E_INVALID, "ddpm_update_peers: null peer array");
+  MKD_REQUIRE(n_peers >= 1 && n_peers <= 8, MKD_E_INVALID, "ddpm_update_peers: n_peers=%d must be 1..8 (one box)",
+              n_peers);
+  PeerPtrs pp = {};
+  for (int r = 0; r < n_peers; ++r) pp.p[r] = x_prev_peers[r];  // host array of device pointers
+  DdpmTables tb = {sqrt_recip_ac, sqrt_recipm1_ac, coef1, coef2, sigma};
+  return ddpm_launch(x, eps, t, B, tb, T, clip, noise, temperature, x0_out, pp, n_peers, n, stream,
+                     "ddpm_update_peers");
 }
 
 // ---------------------------------------------------------------------------------------------------------

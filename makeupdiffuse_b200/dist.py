@@ -14,7 +14,8 @@ only data-path collective is ONE all-gather of the final latents over NVLink 5 /
 ``sample_sharded`` runs the DDIM sampling loop this way; ``encode_sharded`` the DDIM inversion (x_0 -> x_t) of a
 dataset's latents, whose last inversion step writes into the gather buffer the same way; ``sample_plms_sharded`` the PLMS
 sampling loop (B200PLMSSampler), whose last update kernel (``mkd_plms_update[_peers]``) does the same;
-``sample_dpm_sharded`` the DPM-Solver++ loop (B200DPMSolverSampler, ``mkd_dpm_update[_peers]``) likewise.
+``sample_dpm_sharded`` the DPM-Solver++ loop (B200DPMSolverSampler, ``mkd_dpm_update[_peers]``) likewise;
+``sample_ddpm_sharded`` the DDPM ancestral loop (B200DDPMSampler, ``mkd_ddpm_update[_peers]``).
 """
 from __future__ import annotations
 
@@ -126,6 +127,26 @@ def sample_dpm_sharded(sampler, S, batch_global, shape, cond_local, x_T_local, r
     Arguments as sample_sharded; kw goes to sample (guidance).  Returns the [batch_global, C, H, W] latents on every rank.
     Requires equal chunk sizes when world > 1."""
     return _sample_with_sharded(sampler, S, batch_global, shape, cond_local, x_T_local, rank, world, group, fused_gather, kw)
+
+
+def sample_ddpm_sharded(sampler, batch_global, shape, cond_local, x_T_local, rank=0, world=1, group=None, fused_gather=False,
+                        **kw):
+    """DDPM-sample this rank's chunk (B200DDPMSampler.p_sample_loop) and all-gather the final latents.
+
+    shape: one sample's (C, H, W).  Every step, every rank draws the noise of the WHOLE batch, randn((batch_global,
+    *shape)), and keeps its own rows [lo, hi) (x_T too when x_T_local is None): the gathered result is then the
+    single-process result over the global batch, whatever the world size (DESIGN §6); each rank then draws 16 KiB per
+    sample of the whole batch per step at 32 x 32 latents.  That requires every rank's generator to be seeded alike
+    (torch.manual_seed(seed) on each rank before the call).  kw goes to p_sample_loop (timesteps, start_T, callbacks);
+    a mask is not supported.  Returns the [batch_global, C, H, W] latents on every rank.  Requires equal chunk sizes
+    when world > 1."""
+    lo, hi = shard_bounds(batch_global, rank, world)
+    device = sampler.model.device if x_T_local is None else x_T_local.device
+    gathered, mine, hdl, peer_ptrs = _gather_begin(batch_global, lo, hi, tuple(shape), device, world, group, fused_gather)
+    kw.setdefault("verbose", False)
+    sampler.p_sample_loop(cond_local, (hi - lo, *shape), x_T=x_T_local, out=mine, peer_ptrs=peer_ptrs,
+                          noise_rows=(batch_global, lo, hi), **kw)
+    return _gather_end(gathered, mine, hdl, world, group)
 
 
 def encode_sharded(sampler, t_enc, batch_global, x0_local, cond_local, rank=0, world=1, group=None, fused_gather=False,

@@ -147,6 +147,32 @@ def dpm_update(x, eps, x_prev, *, alpha_s, sigma_s, sigma_ratio, phi, order=1, m
     L.check(L.load().mkd_dpm_update(*head, x_prev.data_ptr(), n, _stream()), "dpm_update")
 
 
+def ddpm_update(x, eps, t, x_prev, *, tables, noise, clip, temperature=1.0, x0_out=None, peer_ptrs=None):
+    """One DDPM ancestral step (upstream ddpm.py p_sample after its model call): x, eps, noise [B, ...]; t the B rows'
+    timesteps (int64, on the device); tables [5, T] fp32 rows sqrt_recip_alphas_cumprod, sqrt_recipm1_alphas_cumprod,
+    posterior_mean_coef1, posterior_mean_coef2 and sigma = exp(0.5 * posterior_log_variance_clipped).  The clamped (when
+    clip) x_recon goes to x0_out when given (mkd_ddpm_update in include/mkd_b200.h)."""
+    n, B = x.numel(), x.shape[0]
+    for v in (x, eps, x_prev, noise, x0_out, tables):
+        if v is not None and (v.dtype != torch.float32 or not v.is_contiguous() or not v.is_cuda):
+            raise ValueError("ddpm_update works on contiguous fp32 CUDA latents and tables")
+    for v in (eps, x_prev, noise, x0_out):
+        if v is not None and v.numel() != n:
+            raise ValueError("ddpm_update: every latent-sized tensor must hold x.numel() values")
+    if t.dtype != torch.int64 or t.shape != (B,) or not t.is_contiguous() or not t.is_cuda:
+        raise ValueError("ddpm_update: t must be a contiguous int64 CUDA vector of one timestep per row")
+    if tables.dim() != 2 or tables.shape[0] != 5:
+        raise ValueError("ddpm_update: tables must be [5, T]")
+    T = tables.shape[1]
+    head = (x.data_ptr(), eps.data_ptr(), t.data_ptr(), B, *[tables[k].data_ptr() for k in range(5)], T, int(bool(clip)),
+            noise.data_ptr(), float(temperature), _p(x0_out))
+    if peer_ptrs is not None:  # x_prev goes to every rank's gather buffer (mkd_ddpm_update_peers); x_prev = own slice
+        arr = (C.c_void_p * len(peer_ptrs))(*[int(p) for p in peer_ptrs])
+        L.check(L.load().mkd_ddpm_update_peers(*head, arr, len(peer_ptrs), n, _stream()), "ddpm_update_peers")
+        return
+    L.check(L.load().mkd_ddpm_update(*head, x_prev.data_ptr(), n, _stream()), "ddpm_update")
+
+
 @_timed("nchw_to_nhwc", lambda s, d: _nb(s, d))
 def nchw_to_nhwc(src, dst2d):
     N, Cc, H, W = src.shape

@@ -11,7 +11,8 @@ The RNG stream is consumed exactly like the reference: one ``randn(x.shape)`` pe
 
 ``B200PLMSSampler`` (below) is the drop-in for upstream ``PLMSSampler`` on the same machinery, with its own fused update
 kernel (mkd_plms_update); ``B200DPMSolverSampler`` the drop-in for upstream ``DPMSolverSampler`` (DPM-Solver++(2M) at
-fractional model times, one fused mkd_dpm_update per evaluation).
+fractional model times, one fused mkd_dpm_update per evaluation); ``B200DDPMSampler`` upstream ``LatentDiffusion``'s own
+DDPM ancestral loop (``sample`` / ``p_sample_loop`` / ``progressive_denoising``, one fused mkd_ddpm_update per step).
 """
 from __future__ import annotations
 
@@ -620,3 +621,157 @@ class B200DPMSolverSampler(B200DDIMSampler):
                            peer_ptrs=peer_ptrs if last else None, **st)
             x = x_next
         return x.to(dev), None
+
+
+def _slice_cond(cond, b):
+    """upstream LatentDiffusion.sample's ``cond[:batch_size]`` on every leaf; a None leaf (this model's c_concat may be
+    None) stays None"""
+    cut = lambda v: None if v is None else v[:b]  # noqa: E731
+    if isinstance(cond, dict):
+        return {k: list(map(cut, v)) if isinstance(v, list) else cut(v) for k, v in cond.items()}
+    if isinstance(cond, list):
+        return [cut(v) for v in cond]
+    return cut(cond)
+
+
+class B200DDPMSampler(B200DDIMSampler):
+    """DDPM ancestral sampling, upstream ``ldm.models.diffusion.ddpm.LatentDiffusion``'s ``sample`` / ``p_sample_loop`` /
+    ``progressive_denoising`` / ``p_sample`` lifted onto the B200 machinery; ``B200ControlLDM`` delegates its methods of
+    those names here.  The model supplies upstream's buffers (``sqrt_recip_alphas_cumprod``,
+    ``sqrt_recipm1_alphas_cumprod``, ``posterior_mean_coef1`` / ``2``, ``posterior_log_variance_clipped``) and attributes
+    (``clip_denoised``, ``log_every_t``, ``channels``, ``image_size``, ``q_sample``).  Per step: one graph-replayed
+    UNet+ControlNet call at the integer timestep (the embeddings of all of a loop's timesteps computed up front), one
+    ``randn(x.shape)`` as upstream draws it, also at t = 0, then one fused kernel (mkd_ddpm_update) for x_recon, the clamp,
+    the posterior mean and the noise term.  No classifier-free guidance: upstream's loop has none."""
+
+    def __init__(self, model, schedule="linear", use_cuda_graph=True, **kwargs):
+        super().__init__(model, schedule=schedule, use_cuda_graph=use_cuda_graph, **kwargs)
+        self._ddpm_tables = None
+
+    def _tables(self):
+        """[5, T] fp32 on the model's device: sqrt_recip_ac, sqrt_recipm1_ac, coef1, coef2 and
+        sigma = exp(0.5 * posterior_log_variance_clipped), the last evaluated by torch on the device as upstream does per
+        step (one element at a time on the CPU, see _elementwise)"""
+        if self._ddpm_tables is None:
+            m = self.model
+            f = lambda v: v.to(device=m.device, dtype=torch.float32)  # noqa: E731
+            sigma = _elementwise(lambda v: (0.5 * v).exp(), f(m.posterior_log_variance_clipped))
+            self._ddpm_tables = torch.stack([f(m.sqrt_recip_alphas_cumprod), f(m.sqrt_recipm1_alphas_cumprod),
+                                             f(m.posterior_mean_coef1), f(m.posterior_mean_coef2), sigma]).contiguous()
+        return self._ddpm_tables
+
+    @staticmethod
+    def _randn(shape, device, repeat=False, rows=None):
+        """upstream noise_like(shape, device, repeat).  rows (extension) = (batch_global, lo, hi): draw the noise of the
+        whole batch and keep rows [lo, hi), so a sharded run consumes the RNG as the single-process run does"""
+        if repeat:
+            return torch.randn((1, *shape[1:]), device=device).repeat(shape[0], *((1,) * (len(shape) - 1)))
+        if rows is not None:
+            bg, lo, hi = rows
+            return torch.randn((bg, *shape[1:]), device=device)[lo:hi]
+        return torch.randn(shape, device=device)
+
+    @torch.no_grad()
+    def p_sample(self, x, c, t, clip_denoised=False, repeat_noise=False, return_codebook_ids=False,
+                 quantize_denoised=False, return_x0=False, temperature=1., noise_dropout=0., score_corrector=None,
+                 corrector_kwargs=None, out=None, peer_ptrs=None, t_value=None, noise_rows=None):
+        """upstream p_sample: x_{t-1} (and x_recon when return_x0) from x_t; rows may carry different t.
+        Extensions (optional): ``out`` / ``peer_ptrs`` as in denoising_step; ``t_value`` the timestep as a host int when
+        every row holds it (see _eps); ``noise_rows`` as in _randn."""
+        m = self.model
+        if m.parameterization != "eps":
+            raise NotImplementedError("B200 path implements the yaml's parameterization: eps (yaml:50)")
+        if score_corrector is not None or quantize_denoised or return_codebook_ids:
+            raise NotImplementedError("score_corrector / quantize_denoised / codebook ids are unused by the reference path")
+        x = x.float().contiguous()
+        t = t.to(device=x.device, dtype=torch.int64).contiguous()
+        e = self._eps(x, t, c, t_value)
+        noise = self._randn(x.shape, x.device, repeat_noise, noise_rows)
+        if noise_dropout > 0.:
+            # upstream drops out noise * temperature: the kernel then takes the product as it is
+            noise, temperature = torch.nn.functional.dropout(noise * temperature, p=noise_dropout), 1.
+        x_prev = torch.empty_like(x) if out is None else out
+        x0 = torch.empty_like(x) if return_x0 else None
+        ops.ddpm_update(x, e.contiguous(), t, x_prev, tables=self._tables(), noise=noise.contiguous(), clip=clip_denoised,
+                        temperature=temperature, x0_out=x0, peer_ptrs=peer_ptrs)
+        return (x_prev, x0) if return_x0 else x_prev
+
+    def _loop(self, cond, shape, x_T, timesteps, log_every_t, mask, x0, callback, img_callback, progressive, temperature,
+              out, peer_ptrs, noise_rows, **step):
+        """the loop of p_sample_loop (progressive=False) and progressive_denoising (True); returns (img, intermediates)"""
+        m = self.model
+        if (out is not None or peer_ptrs is not None) and (mask is not None or timesteps < 1):
+            raise ValueError("out= / peer_ptrs= receive the last step's result: they need a step, and no mask blend after it")
+        log_every_t = log_every_t or m.log_every_t
+        b = shape[0]
+        img = self._randn(shape, m.device, rows=noise_rows) if x_T is None else x_T
+        intermediates = [] if progressive else [img]
+        if progressive and type(temperature) == float:  # noqa: E721  (upstream's test: only a float is expanded)
+            temperature = [temperature] * timesteps
+        self.begin_loop(range(timesteps - 1, -1, -1))
+        for i in reversed(range(0, timesteps)):
+            ts = torch.full((b,), i, device=m.device, dtype=torch.long)
+            res = self.p_sample(img, cond, ts, clip_denoised=m.clip_denoised, return_x0=progressive,
+                                temperature=temperature[i] if progressive else 1., t_value=i, noise_rows=noise_rows,
+                                out=out if i == 0 else None, peer_ptrs=peer_ptrs if i == 0 else None, **step)
+            img, x0_partial = res if progressive else (res, None)
+            if mask is not None:
+                assert x0 is not None
+                img = m.q_sample(x0, ts) * mask + (1. - mask) * img  # after the step, with its own draw
+            if i % log_every_t == 0 or i == timesteps - 1:
+                intermediates.append(x0_partial if progressive else img)
+            if callback:
+                callback(i)
+            if img_callback:
+                img_callback(img, i)
+        return img, intermediates
+
+    @torch.no_grad()
+    def p_sample_loop(self, cond, shape, return_intermediates=False, x_T=None, verbose=True, callback=None,
+                      timesteps=None, quantize_denoised=False, mask=None, x0=None, img_callback=None, start_T=None,
+                      log_every_t=None, out=None, peer_ptrs=None, noise_rows=None):
+        """upstream p_sample_loop: img, or (img, intermediates) with the start and every log_every_t-th step.
+        Extensions (optional): ``out`` / ``peer_ptrs`` as in denoising_step, for the LAST step only; ``noise_rows`` as in
+        _randn, for x_T and every step's noise."""
+        if timesteps is None:
+            timesteps = self.model.num_timesteps
+        if start_T is not None:
+            timesteps = min(timesteps, start_T)
+        if mask is not None:
+            assert x0 is not None
+            assert x0.shape[2:3] == mask.shape[2:3]  # sic: upstream compares one spatial dimension
+        img, intermediates = self._loop(cond, shape, x_T, timesteps, log_every_t, mask, x0, callback, img_callback, False,
+                                        1., out, peer_ptrs, noise_rows, quantize_denoised=quantize_denoised)
+        return (img, intermediates) if return_intermediates else img
+
+    @torch.no_grad()
+    def progressive_denoising(self, cond, shape, verbose=True, callback=None, quantize_denoised=False, img_callback=None,
+                              mask=None, x0=None, temperature=1., noise_dropout=0., score_corrector=None,
+                              corrector_kwargs=None, batch_size=None, x_T=None, start_T=None, log_every_t=None):
+        """upstream progressive_denoising: (img, the x_recon of every log_every_t-th step); temperature is a float or one
+        value per timestep, indexed by the timestep"""
+        if batch_size is not None:
+            shape = [batch_size] + list(shape)
+        else:
+            batch_size = shape[0]
+        if cond is not None:
+            cond = _slice_cond(cond, batch_size)
+        timesteps = self.model.num_timesteps
+        if start_T is not None:
+            timesteps = min(timesteps, start_T)
+        return self._loop(cond, shape, x_T, timesteps, log_every_t, mask, x0, callback, img_callback, True, temperature,
+                          None, None, None, quantize_denoised=quantize_denoised, noise_dropout=noise_dropout,
+                          score_corrector=score_corrector, corrector_kwargs=corrector_kwargs)
+
+    @torch.no_grad()
+    def sample(self, cond, batch_size=16, return_intermediates=False, x_T=None, verbose=True, timesteps=None,
+               quantize_denoised=False, mask=None, x0=None, shape=None, **kwargs):
+        """upstream LatentDiffusion.sample (not DDIM's sample(S, ...)): every cond leaf cut to batch_size rows, the
+        default shape (batch_size, model.channels, model.image_size, model.image_size), then p_sample_loop"""
+        m = self.model
+        if shape is None:
+            shape = (batch_size, m.channels, m.image_size, m.image_size)
+        if cond is not None:
+            cond = _slice_cond(cond, batch_size)
+        return self.p_sample_loop(cond, shape, return_intermediates=return_intermediates, x_T=x_T, verbose=verbose,
+                                  timesteps=timesteps, quantize_denoised=quantize_denoised, mask=mask, x0=x0)
