@@ -241,7 +241,8 @@ typedef struct mkd_conv_desc {
   const float* bias;
   const void* emb; /* [N, lde] activations dtype */
   const void* residual;
-  int residual_dtype; /* MKD_BF16 / MKD_F32: storage type of `residual` (fp32 for trunk tensors kept unrounded) */
+  int residual_dtype; /* MKD_BF16 / MKD_F32: storage type of `residual` (fp32 for trunk tensors kept unrounded); with a
+                         residual it must be MKD_F32 when `dtype` is MKD_F32 */
   int ldy32;
   float* y32;         /* optional fp32 copy of the output (same values before rounding); `y` may then be NULL */
   void* workspace; /* split-K partials (tcgen05 path); may be NULL -> no split-K */

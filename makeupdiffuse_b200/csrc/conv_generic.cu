@@ -164,7 +164,7 @@ int conv2d_generic(const mkd_conv_desc* d, cudaStream_t stream) {
   p.gb = d->geglu_block > 0 ? d->geglu_block : 1;
   p.Kout = d->act == MKD_ACT_GEGLU ? d->K / 2 : d->K;
   p.alpha = d->alpha;
-  p.res_f32 = (d->residual_dtype == MKD_F32 || d->dtype == MKD_F32) ? 1 : 0;
+  p.res_f32 = d->residual_dtype == MKD_F32 ? 1 : 0;
   p.y32 = d->y32;
   p.ldy32 = d->ldy32;
   dim3 grid((p.M + BM - 1) / BM, (p.Kout + BN - 1) / BN);
@@ -197,6 +197,8 @@ static int validate(const mkd_conv_desc* d) {
   MKD_REQUIRE(d->dtype == MKD_BF16 || d->dtype == MKD_F32, MKD_E_INVALID, "conv2d: bad dtype %d", d->dtype);
   MKD_REQUIRE(d->x && d->w && (d->y || d->y32), MKD_E_INVALID, "conv2d: null x/w/y");
   MKD_REQUIRE(d->residual_dtype == MKD_BF16 || d->residual_dtype == MKD_F32, MKD_E_INVALID, "conv2d: bad residual_dtype");
+  MKD_REQUIRE(!d->residual || d->dtype == MKD_BF16 || d->residual_dtype == MKD_F32, MKD_E_INVALID,
+              "conv2d: an fp32 conv takes an fp32 residual");
   MKD_REQUIRE(d->N > 0 && d->H > 0 && d->W > 0 && d->C > 0 && d->K > 0 && d->R > 0 && d->S > 0 && d->stride > 0 &&
                   d->pad >= 0 && d->pad_hi_extra >= 0 && d->pad_hi_extra <= 1,
               MKD_E_INVALID, "conv2d: non-positive dimension");

@@ -46,3 +46,20 @@ def test_conv_desc_struct_layout_matches_header():
     assert lib.mkd_conv2d_path(ctypes.byref(d)) == _lib.PATH_GENERIC
     d.path = _lib.PATH_TCGEN05
     assert lib.mkd_conv2d_path(ctypes.byref(d)) < 0 and b"stride" in lib.mkd_last_error()
+
+
+def test_fp32_conv_rejects_a_bf16_residual():
+    """the generic kernel reads an fp32 conv's residual as fp32: a bf16 residual_dtype there is refused, not misread"""
+    MKD_E_INVALID = -1  # include/mkd_b200.h
+    lib = _lib.load()
+    d = _lib.ConvDesc()
+    d.x = d.w = d.y = d.residual = 16
+    d.dtype, d.N, d.H, d.W, d.C, d.K, d.R, d.S, d.stride, d.pad = _lib.MKD_F32, 1, 8, 8, 64, 64, 3, 3, 1, 1
+    d.ldx = d.ldy = d.ldr = 64
+    d.path = _lib.PATH_GENERIC
+    d.residual_dtype = _lib.MKD_F32
+    assert lib.mkd_conv2d_path(ctypes.byref(d)) == _lib.PATH_GENERIC
+    d.residual_dtype = _lib.MKD_BF16
+    assert lib.mkd_conv2d_path(ctypes.byref(d)) == MKD_E_INVALID and b"fp32 residual" in lib.mkd_last_error()
+    d.path = _lib.PATH_AUTO
+    assert lib.mkd_conv2d_path(ctypes.byref(d)) == MKD_E_INVALID

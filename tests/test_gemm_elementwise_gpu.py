@@ -30,8 +30,8 @@ about 8x of the measured maximum over every case here (a run prints the margin),
 k-block (~8 / (0.64 K_tot) >= 4e-4) or a wrong embedding row produces.
 
 Out of scope: MKD_DUAL=1 (variants 10 / 11) and MKD_CLUSTER=2 (the CL = 2 single-CTA kernel) — opt-in experiments, read once
-per process and absent from the shipped library's code path; the generic kernel; weight groups (mkd_conv_desc.wgroups: the
-same pair instantiations, compared with two single-group launches in test_kernels_gpu).
+per process and absent from the shipped library's code path; the generic kernel (test_conv_generic_elementwise_gpu.py); weight
+groups (mkd_conv_desc.wgroups: the same pair instantiations, compared with two single-group launches in test_kernels_gpu).
 """
 import math
 import re
@@ -48,6 +48,8 @@ from test_kernels_gpu import GN_TAIL_CASES, PAIR_CASES, PAIR_STATS_CASES
 U = 2.0 ** -24
 TAU_STATS = 2.0 ** -17           # fp32 sum of <= 128 values in any order: |err| <= 127 u sum |v|
 GELU_APPROX = 0.75e-7 + 2.0 ** -22  # common.cuh: erf by A-S 7.1.26 (0.75e-7 |x| on gelu) + rcp / ex2.approx and fp32 steps
+GELU_ERFF = 2.0 ** -22           # gelu_erf_f (generic kernel): erff 2 ulp + 1 + erf and the product rounded: <= 3 u |x|
+SILU_FLUSH = 2.0 ** -119         # silu_f returns 0 once 1 + e^-x > 2^126 (x < -87.3), where |silu(x)| < 2^7 2^-126
 BF16_REL = 2.0 ** -8             # bf16 unit roundoff: 8 significant bits
 WS_BYTES = 64 << 20
 NAN = float("nan")
@@ -56,17 +58,24 @@ MEASURED = {"err_over_A": (0.0, ""), "c": (0.0, ""), "gelu_coef": (0.0, "")}  # 
 #                                                                            worst GELU approximation error implied per |a| |g|
 
 
+def depth(s):
+    """K_tot = R S C + C2: the contraction length"""
+    return s["R"] * s["R"] * s["C"] + s["C2"]
+
+
 def tau(s):
-    """per-element accumulation bound relative to A (module docstring)"""
-    return U * math.sqrt(s["R"] * s["R"] * s["C"] + s["C2"])
+    """per-element accumulation bound relative to A: u sqrt(K_tot) (module docstring); for the generic kernel's serial fmaf
+    chain 2 u sqrt(K_tot + 4) (test_conv_generic_elementwise_gpu.py)"""
+    return 2 * U * math.sqrt(depth(s) + 4) if s["generic"] else U * math.sqrt(depth(s))
 
 
 # ---- float64 reference ----------------------------------------------------------------------------------------------------
 def spec_of(**s):
-    """a case: conv geometry + operand set.  res: None / "bf16" / "f32"; inplace: the residual is the output of its dtype"""
+    """a case: conv geometry + operand set.  res: None / "bf16" / "f32"; inplace: the residual is the output of its dtype;
+    dtype: "bf16" / "f32" (x, w, emb, y); generic: the case runs on the generic kernel (its accumulation and GELU bounds)"""
     d = dict(N=1, H=1, W=1, C=64, K=64, R=1, stride=1, pad=None, pad_hi_extra=0, up=False, bias=True, spread=0.0, emb=False,
              res=None, inplace=False, alpha=1.0, act="none", gb=80, y=True, y32=False, stats=False, ws=False, C2=0, tight=False,
-             gn=None, exact=False)
+             gn=None, exact=False, dtype="bf16", generic=False)
     d.update(s)
     if d["pad"] is None:
         d["pad"] = d["R"] // 2
@@ -110,8 +119,9 @@ def reference(s, x, w, bias, emb, res, x2):
         ref = a * ga
         ea, eg = t * Aa, t * Ag
         op = ga.abs() * ea + 1.13 * (a.abs() + ea) * eg              # the operands' own errors, through the product
-        b16 = BF16_REL * ref.abs() + (1 + BF16_REL) * (op + (a.abs() + ea) * GELU_APPROX * (g.abs() + eg))
-        return dict(ref=ref, b32=None, b16=b16, geglu=(a, g, ea, eg, op))
+        ge = op + (a.abs() + ea) * (GELU_ERFF if s["generic"] else GELU_APPROX) * (g.abs() + eg)
+        return dict(ref=ref, b32=U * ref.abs() + (1 + U) * ge, b16=BF16_REL * ref.abs() + (1 + BF16_REL) * ge,
+                    geglu=(a, g, ea, eg, op))
     pre = acc + b
     A = mag + b.abs()
     if emb is not None:
@@ -123,7 +133,7 @@ def reference(s, x, w, bias, emb, res, x2):
     if s["act"] == "silu":
         ref = F.silu(pre)
         # __expf: 2 + 1.17 |x| ulp, __fdividef: 2 ulp, the 1 + e rounding: 1/2 ulp (CUDA C Programming Guide, intrinsics)
-        b32 = 1.1 * t * A + (5.0 + 1.2 * pre.abs()) * 2.0 ** -23 * ref.abs()
+        b32 = 1.1 * t * A + (5.0 + 1.2 * pre.abs()) * 2.0 ** -23 * ref.abs() + SILU_FLUSH
     else:
         ref, b32 = pre, t * A
     return dict(ref=ref, b32=b32, b16=BF16_REL * ref.abs() + (1 + BF16_REL) * b32, A=A, pre=pre)
@@ -178,6 +188,26 @@ def check_outputs(label, s, refd, y=None, y32=None, stats=None, guards=(), gn=No
     ref = refd["ref"]
     worst = {}
     check_guards(guards)
+
+    def measure(err, rel):
+        if s["act"] == "none":
+            r, at = _worst(err, refd["A"])
+            if r > MEASURED["err_over_A"][0]:
+                MEASURED["err_over_A"] = (r, label)
+            if r / (U * math.sqrt(depth(s))) > MEASURED["c"][0]:
+                MEASURED["c"] = (r / (U * math.sqrt(depth(s))), label)
+        if "geglu" in refd:  # the GELU approximation error this output implies (what rounding and operands cannot explain)
+            a, g, ea, eg, op = refd["geglu"]
+            excess = (err - rel * (ref.abs() + op) - op) / (1 + rel)
+            coef = float((excess / ((a.abs() + ea) * (g.abs() + eg)).clamp_min(1e-30)).max())
+            if coef > MEASURED["gelu_coef"][0]:
+                MEASURED["gelu_coef"] = (coef, label)
+
+    def exact(name, got, dtype):
+        """exact operands, no activation: every partial sum is representable, so the output is ref rounded once"""
+        if s["exact"] and s["act"] == "none":
+            want = ref.to(dtype).double()
+            assert torch.equal(got, want), f"{label}: {name} != ref rounded to {dtype} at {(got != want).nonzero()[0].tolist()}"
     if y32 is not None:
         got = y32.double()
         assert bool(torch.isfinite(got).all()), f"{label}: y32 holds {int((~torch.isfinite(got)).sum())} non-finite values"
@@ -185,29 +215,26 @@ def check_outputs(label, s, refd, y=None, y32=None, stats=None, guards=(), gn=No
         worst["y32"], at = _worst(err, refd["b32"])
         assert worst["y32"] <= 1.0, (f"{label}: y32[{at}] = {float(got[at]):.9g}, reference {float(ref[at]):.9g}, |err| / bound "
                                      f"{worst['y32']:.3g}")
-        if s["act"] == "none":
-            r, at = _worst(err, refd["A"])
-            if r > MEASURED["err_over_A"][0]:
-                MEASURED["err_over_A"] = (r, label)
-            if r / tau(s) > MEASURED["c"][0]:
-                MEASURED["c"] = (r / tau(s), label)
+        exact("y32", got, torch.float32)
+        measure(err, U)
     if y is not None:
         got = y.double()
+        f32 = y.dtype == torch.float32
         assert bool(torch.isfinite(got).all()), f"{label}: y holds {int((~torch.isfinite(got)).sum())} non-finite values"
-        if y32 is not None:
+        if y32 is not None and f32:  # one fp32 value stored twice
+            same = _bits(y) == _bits(y32)
+            assert bool(same.all()), f"{label}: y != y32 bit for bit at {(~same).nonzero()[0].tolist()}"
+        elif y32 is not None:
             same = y == y32.to(torch.bfloat16)
             assert bool(same.all()), f"{label}: y != bf16(y32) at {(~same).nonzero()[0].tolist()}"
         else:
             err = (got - ref).abs()
-            worst["y"], at = _worst(err, refd["b16"])
-            assert worst["y"] <= 1.0, (f"{label}: y[{at}] = {float(got[at]):.6g}, reference {float(ref[at]):.6g}, |err| / bound "
+            worst["y"], at = _worst(err, refd["b32" if f32 else "b16"])
+            assert worst["y"] <= 1.0, (f"{label}: y[{at}] = {float(got[at]):.9g}, reference {float(ref[at]):.9g}, |err| / bound "
                                        f"{worst['y']:.3g}")
-            if "geglu" in refd:  # the GELU approximation error this output implies (what rounding and operands cannot explain)
-                a, g, ea, eg, op = refd["geglu"]
-                excess = (err - BF16_REL * (ref.abs() + op) - op) / (1 + BF16_REL)
-                coef = float((excess / ((a.abs() + ea) * (g.abs() + eg)).clamp_min(1e-30)).max())
-                if coef > MEASURED["gelu_coef"][0]:
-                    MEASURED["gelu_coef"] = (coef, label)
+            exact("y", got, y.dtype)
+            if f32 or "geglu" in refd:
+                measure(err, U if f32 else BF16_REL)
     if stats is not None:
         Mo, K = ref.shape
         T = stats.shape[0]
@@ -240,11 +267,9 @@ def check_outputs(label, s, refd, y=None, y32=None, stats=None, guards=(), gn=No
 
 # ---- buffers ----------------------------------------------------------------------------------------------------------------
 def guarded(rows, cols, dtype, device, tight=False, extra_rows=3):
-    """NaN-filled buffer holding a [rows, cols] view: 8 guard columns on each side (ld a multiple of 8) unless tight"""
+    """NaN-filled buffer holding a [rows, cols] view: 8 guard columns on each side (ld a multiple of 8) unless tight (ld = cols)"""
     off = 0 if tight else 8
     ld = off + cols + (0 if tight else 8 + (-(off + cols)) % 8)
-    if tight and ld % 8:
-        ld += (-ld) % 8
     buf = torch.full((rows + extra_rows, ld), NAN, dtype=dtype, device=device)
     return buf, buf[:rows, off:off + cols], (slice(0, rows), slice(off, off + cols))
 
@@ -258,24 +283,28 @@ def make_operands(s, device, seed):
     P, Q, Mo = out_geometry(s)
     Ko = K // 2 if s["act"] == "geglu" else K
     BF, F32 = torch.bfloat16, torch.float32
+    AT = {"bf16": BF, "f32": F32}[s["dtype"]]  # x, w, emb, y
     bufs = {}
 
     def put(name, rows, cols, dtype, fill, tight=None):
-        buf, view, inside = guarded(rows, cols, dtype, device, tight=s["tight"] if tight is None else tight)
+        if tight is None:  # s["tight"]: True / False for every view, or the names of the views that are tight
+            tight = s["tight"] if isinstance(s["tight"], bool) else name in s["tight"]
+        buf, view, inside = guarded(rows, cols, dtype, device, tight=tight)
         if fill is not None:
             view.copy_(fill)
         bufs[name] = (buf, inside)
         return view
     fan = R * R * C + s["C2"]
     ints = lambda lo, hi, *shape: torch.randint(lo, hi + 1, shape, device=device, generator=g).float()  # noqa: E731
-    if s["exact"]:  # x in {-2..2}, w in 2^-7 {-8..8}, bias in 2^-7 {-1024..1024}: every partial sum is k 2^-7, |k| < 2^24
-        assert not s["C2"] and not s["emb"] and s["res"] is None and 2 * 8 * fan + 1024 < 2 ** 24
-        x = put("x", N * H * W, C, BF, ints(-2, 2, N * H * W, C))
-        w = (ints(-8, 8, K, fan) / 128).to(BF)
+    if s["exact"]:  # x in {-2..2}, w in 2^-7 {-8..8}, bias in 2^-7 {-1024..1024}, emb in 2^-7 {-256..256}, residual in
+        # 2^-8 {-256..256} (bf16 holds integers up to 256), alpha in {0.5, 1, 2}: every partial sum is k 2^-8, |k| < 2^24
+        assert not s["C2"] and s["alpha"] in (0.5, 1.0, 2.0) and 2 * 2 * (16 * fan + 1024 + 256) + 256 < 2 ** 24
+        x = put("x", N * H * W, C, AT, ints(-2, 2, N * H * W, C))
+        w = (ints(-8, 8, K, fan) / 128).to(AT)
     else:
-        x = put("x", N * H * W, C, BF, rnd(N * H * W, C))
-        w = (rnd(K, fan) / math.sqrt(fan)).to(BF)
-    x2 = put("x2", N * H * W, s["C2"], BF, rnd(N * H * W, s["C2"])) if s["C2"] else None
+        x = put("x", N * H * W, C, AT, rnd(N * H * W, C))
+        w = (rnd(K, fan) / math.sqrt(fan)).to(AT)
+    x2 = put("x2", N * H * W, s["C2"], AT, rnd(N * H * W, s["C2"])) if s["C2"] else None
     if not s["bias"]:
         bias = None
     elif s["exact"]:
@@ -284,16 +313,20 @@ def make_operands(s, device, seed):
         bias = (torch.rand(K, device=device, generator=g) * 2 - 1) * s["spread"]
     else:
         bias = 0.5 * rnd(K)
-    emb = put("emb", N, K, BF, rnd(N, K), tight=False) if s["emb"] else None
-    y = put("y", Mo, Ko, BF, rnd(Mo, Ko) if (s["inplace"] and s["res"] == "bf16") else None) if s["y"] else None
-    y32 = put("y32", Mo, Ko, F32, rnd(Mo, Ko) if (s["inplace"] and s["res"] == "f32") else None) if s["y32"] else None
+    emb = put("emb", N, K, AT, ints(-256, 256, N, K) / 128 if s["exact"] else rnd(N, K), tight=False) if s["emb"] else None
+    resv = lambda: ints(-256, 256, Mo, Ko) / 256 if s["exact"] else rnd(Mo, Ko)  # noqa: E731
+    # an in-place residual is the output of its dtype: y when that is y's dtype (and y is written), else y32
+    into_y = s["inplace"] and s["y"] and s["res"] == s["dtype"]
+    y = put("y", Mo, Ko, AT, resv() if into_y else None) if s["y"] else None
+    y32 = put("y32", Mo, Ko, F32, resv() if (s["inplace"] and s["res"] == "f32" and not into_y) else None) if s["y32"] else None
     if s["res"] is None:
         res = None
     elif s["inplace"]:
-        res = y if s["res"] == "bf16" else y32
-        assert res is not None, "an in-place residual needs the output of its dtype"
+        res = y if into_y else y32
+        assert res is not None and res.dtype == {"bf16": BF, "f32": F32}[s["res"]], \
+            "an in-place residual needs the output of its dtype"
     else:
-        res = put("res", Mo, Ko, BF if s["res"] == "bf16" else F32, rnd(Mo, Ko))
+        res = put("res", Mo, Ko, BF if s["res"] == "bf16" else F32, resv())
     stats = None
     if s["stats"]:
         T = (Mo + 127) // 128
